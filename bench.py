@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark of the self-play hot path (BASELINE.json metric).
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            own arm (CUDA kernels + bf16 net)
+  python bench.py ... --dump-outputs DIR                         also write the last timed move's samples as .npy
   python bench.py --impl reference [--steps K] [--warmup W]      reference arm (CPU port of collect.py)
   torchrun --nproc-per-node N ... bench.py --gpus N ...          one rank per GPU, games sharded
 
@@ -73,7 +74,15 @@ def parse_args():
     ap.add_argument("--conv-impl", default=None, choices=["k9", "k9_skip", "cudnn"],
                     help="tower convolution kernel (default: the evaluator's default, K9 = csrc/ccz_conv.cuh)")
     ap.add_argument("--conv-sample", type=int, default=8, help="bracket every K9 launch of every n-th forward with CUDA events")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the samples of the last timed move of the `value` arm as DIR/<name>.npy (float32 / "
+                         "float64, rank 0, at most 64 MB: a fixed seeded subset of the games beyond that)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "own":
+        ap.error("--dump-outputs needs --impl own")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -133,6 +142,28 @@ def measured_peaks():
         return {"hbm_gbs": p["hbm_gbs"], "bf16_tflops": p["bf16_tflops"],
                 "bf16_tflops_sustained": p.get("bf16_tflops_sustained", p["bf16_tflops"]), "source": "measured"}
     return {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0, "source": "fallback"}
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir: str, sample: dict, limit: int = DUMP_LIMIT) -> None:
+    """One move's per-game samples (SelfPlayEngine.drain_resident() keys, one row per game) as float32 / float64
+    .npy files, so that two builds can be compared output for output.  ``game_index.npy`` names the games kept:
+    all of them, or a fixed seeded subset when the files would exceed ``limit`` bytes."""
+    import numpy as np
+
+    arrays = {k: v.astype(np.float64 if v.dtype == np.float64 else np.float32) for k, v in sample.items()}
+    n_games = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(a[0].nbytes for a in arrays.values()) + 8  # + the float64 game index
+    budget = limit - 128 * (len(arrays) + 1)  # an .npy header of these shapes is 128 bytes
+    games = np.arange(n_games)
+    if row_bytes * n_games > budget:
+        games = np.sort(np.random.default_rng(0).choice(n_games, budget // row_bytes, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "game_index.npy"), games.astype(np.float64))
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a[games])
 
 
 # ------------------------------------------------------------------------------------------------
@@ -459,6 +490,10 @@ def run_own_arm(args):
     dev_ms = max_over_ranks(s0_s1_ms)
     value = world * G * args.steps / dev_ms * 1e3
     resident_samples = sum(int(d["boards"].shape[0]) for d in eng.resident_backlog) * G
+    if args.dump_outputs and rank == 0:
+        # a ring that filled with the last move was drained inside it, leaving the final drain empty
+        last = next(d for d in reversed(eng.resident_backlog) if d["boards"].shape[0])
+        dump_outputs(args.dump_outputs, {k: v[-1] for k, v in last.items()})
     pool_value = eng.pool_events()
     # K3 for `roofline.mcts`: 64 more playouts so that the trees are a few levels deep, then 50 launches in one event
     # bracket (select only reads the trees and writes the leaf scratch buffers)

@@ -22,7 +22,7 @@ def _step(device_is_gpu):
 
     states, probs, winners = train_batch()
     torch.manual_seed(0)
-    pipe = TrainPipeline(batch_size=len(states))
+    pipe = TrainPipeline(batch_size=len(states), net_kwargs=dict(use_gpu=device_is_gpu))
     assert pipe.policy_value_net.device.type == ("cuda" if device_is_gpu else "cpu")
     r = pipe.train_step(torch.tensor(states, dtype=torch.float32), torch.tensor(probs, dtype=torch.float32),
                         torch.tensor(winners, dtype=torch.float32))
@@ -34,7 +34,6 @@ def _step(device_is_gpu):
     return pipe, r
 
 
-@pytest.mark.skipif(torch.cuda.is_available(), reason="CPU fp32 parity runs where no GPU is visible")
 def test_cpu_fp32_step_matches_reference(gold):
     pipe, r = _step(False)
     g = gold["log"]
