@@ -29,6 +29,7 @@ CTL_HEAD, CTL_TAIL, CTL_EXPAND_FAILED, CTL_TREES_DROPPED, CTL_MIN_FREE, CTL_WORD
 NODE_BYTES = 24  # ccz_node (16) + ccz_link (8)
 MAX_CHILDREN = 119  # most legal moves of any Xiangqi position
 POLICY_PROBS, POLICY_LOGITS = 0, 1
+DEDUP_MAX_BOARDS = 16384  # largest leaf batch ccz_leaf_unique takes
 CONV_VARIANT_1CTA, CONV_VARIANT_PAIR, CONV_VARIANT_2PAIRS, CONV_VARIANT_4PAIRS = 1, 2, 2 | 32, 2 | 64
 
 EXPORTS = (
@@ -37,7 +38,7 @@ EXPORTS = (
     "ccz_movegen_encode", "ccz_board_keys_init", "ccz_board_push", "ccz_mcts_pool_init", "ccz_mcts_reset",
     "ccz_mcts_reserve", "ccz_mcts_migrate", "ccz_mcts_select",
     "ccz_mcts_expand_backup", "ccz_mcts_root_visits", "ccz_mcts_advance", "ccz_replay_pack", "ccz_conv3x3_c256", "ccz_conv3x3_plan", "ccz_stem_lookup",
-    "ccz_heads_pack",
+    "ccz_heads_pack", "ccz_conv3x3_c256_count", "ccz_stem_lookup_count", "ccz_heads_pack_rows", "ccz_leaf_unique",
 )
 
 
@@ -122,6 +123,10 @@ def load() -> ctypes.CDLL:
     lib.ccz_stem_lookup.argtypes = [vp, i32, vp, vp, vp, vp]
     lib.ccz_conv3x3_plan.argtypes = [i32, i32, i32, vp]
     lib.ccz_heads_pack.argtypes = [vp, i32, vp, i32, i32, vp]
+    lib.ccz_conv3x3_c256_count.argtypes = [vp, vp, vp, vp, vp, i32, vp, i32, vp]
+    lib.ccz_stem_lookup_count.argtypes = [vp, i32, vp, vp, vp, vp, vp]
+    lib.ccz_heads_pack_rows.argtypes = [vp, i32, vp, vp, i32, i32, vp]
+    lib.ccz_leaf_unique.argtypes = [vp, i32, vp, vp, vp, vp, vp]
     for name in EXPORTS:
         if name not in ("ccz_last_error",):
             getattr(lib, name).restype = i32
@@ -391,14 +396,21 @@ def replay_pack(hist_boards, turn_plane, acts, probs, counts):
     return states, pi
 
 
+def _check_count(count: torch.Tensor, dev) -> None:
+    if count.dtype != torch.int32 or count.numel() != 1 or count.device != dev:
+        raise CczError("count must be a one-element int32 tensor on the boards' device")
+
+
 def conv3x3_c256(x: torch.Tensor, w: torch.Tensor, bias: torch.Tensor, skip: torch.Tensor | None = None,
-                 out: torch.Tensor | None = None, variant: int = 0) -> torch.Tensor:
+                 out: torch.Tensor | None = None, variant: int = 0, count: torch.Tensor | None = None) -> torch.Tensor:
     """K9: relu(conv3x3_pad1(x, w) + bias [+ skip]) on the tcgen05 tensor cores.
 
     ``x`` / ``skip`` / ``out``: bf16 ``(n,256,10,9)`` tensors in ``torch.channels_last`` memory
     format (= NHWC rows of 256 channels); ``w``: bf16 ``(256,256,3,3)`` channels_last; ``bias`` fp32 (256,).
     ``variant`` 0 = the library default; other values select the tiling for measurements
     (``CONV_VARIANT_*``: 1 single-CTA tiles, 2 CTA pairs, 34 / 66 clusters of 2 / 4 pairs sharing weight stages).
+    ``count``: int32 (1,) device tensor -- only the first ``count`` boards are convolved (``ccz_conv3x3_c256_count``);
+    the later rows of ``out`` are left unspecified.
     """
     cl = torch.channels_last
     if x.dtype != torch.bfloat16 or w.dtype != torch.bfloat16 or bias.dtype != torch.float32:
@@ -417,19 +429,24 @@ def conv3x3_c256(x: torch.Tensor, w: torch.Tensor, bias: torch.Tensor, skip: tor
         raise CczError("conv3x3_c256: variant out of range (see ccz_conv3x3_c256 in include/ccz_b200.h)")
     if not (x.is_cuda and w.is_cuda and bias.is_cuda and out.is_cuda):
         raise CczError("device tensor expected (the C ABI takes device pointers)")
+    sk = None if skip is None else skip.data_ptr()
     with torch.cuda.device(x.device):
-        check(
-            load().ccz_conv3x3_c256(x.data_ptr(), w.data_ptr(), bias.data_ptr(), None if skip is None else skip.data_ptr(),
-                                    out.data_ptr(), int(x.shape[0]), int(variant), stream_ptr(x.device)),
-            "ccz_conv3x3_c256",
-        )
+        if count is None:
+            check(load().ccz_conv3x3_c256(x.data_ptr(), w.data_ptr(), bias.data_ptr(), sk, out.data_ptr(), int(x.shape[0]),
+                                          int(variant), stream_ptr(x.device)), "ccz_conv3x3_c256")
+        else:
+            _check_count(count, x.device)
+            check(load().ccz_conv3x3_c256_count(x.data_ptr(), w.data_ptr(), bias.data_ptr(), sk, out.data_ptr(), int(x.shape[0]),
+                                                count.data_ptr(), int(variant), stream_ptr(x.device)), "ccz_conv3x3_c256_count")
     return out
 
 
-def stem_lookup(boards: torch.Tensor, table: torch.Tensor, bias_turn: torch.Tensor, out: torch.Tensor | None = None) -> torch.Tensor:
+def stem_lookup(boards: torch.Tensor, table: torch.Tensor, bias_turn: torch.Tensor, out: torch.Tensor | None = None,
+                count: torch.Tensor | None = None) -> torch.Tensor:
     """K10: stem conv + BN + ReLU of search-time inputs straight from ``boards`` (n,96) uint8 ->
     bf16 ``(n,256,10,9)`` channels_last.  ``table`` bf16 (9,16,256), ``bias_turn`` fp32 (2,9,256)
-    (built by ``net.stem_tables``)."""
+    (built by ``net.stem_tables``).  ``count``: int32 (1,) device tensor -- only the first ``count`` boards
+    are evaluated (``ccz_stem_lookup_count``), later output rows are not written."""
     n = boards.shape[0]
     if boards.dtype != torch.uint8 or boards.shape[1:] != (BOARD_BYTES,):
         raise CczError("stem_lookup: boards must be uint8 (n,96)")
@@ -441,21 +458,52 @@ def stem_lookup(boards: torch.Tensor, table: torch.Tensor, bias_turn: torch.Tens
     elif tuple(out.shape) != (n, 256, 10, 9) or out.dtype != torch.bfloat16 or not out.is_contiguous(memory_format=torch.channels_last):
         raise CczError("stem_lookup: out must be bf16 (n,256,10,9) channels_last")
     with torch.cuda.device(boards.device):
-        check(load().ccz_stem_lookup(_ptr(boards), n, _ptr(table), _ptr(bias_turn), out.data_ptr(), stream_ptr(boards.device)),
-              "ccz_stem_lookup")
+        if count is None:
+            check(load().ccz_stem_lookup(_ptr(boards), n, _ptr(table), _ptr(bias_turn), out.data_ptr(), stream_ptr(boards.device)),
+                  "ccz_stem_lookup")
+        else:
+            _check_count(count, boards.device)
+            check(load().ccz_stem_lookup_count(_ptr(boards), n, count.data_ptr(), _ptr(table), _ptr(bias_turn), out.data_ptr(),
+                                               stream_ptr(boards.device)), "ccz_stem_lookup_count")
     return out
 
 
-def heads_pack(h: torch.Tensor, operands: torch.Tensor, value_off: int) -> torch.Tensor:
+def heads_pack(h: torch.Tensor, operands: torch.Tensor, value_off: int, rows: torch.Tensor | None = None) -> torch.Tensor:
     """K11: ``h`` bf16 (n*90, 32) head-convolution outputs (bias added, before the ReLU) -> ``operands`` bf16 (n, K)
-    with relu(policy) channel-major at column 0 and relu(value) at column ``value_off`` (net.py:96-97,103-104)."""
+    with relu(policy) channel-major at column 0 and relu(value) at column ``value_off`` (net.py:96-97,103-104).
+    ``rows``: int32 (n,) device tensor -- operand row b is packed from board ``rows[b]`` of ``h`` (``ccz_heads_pack_rows``);
+    the caller guarantees every entry is below n."""
     n = operands.shape[0]
     if h.dtype != torch.bfloat16 or operands.dtype != torch.bfloat16 or tuple(h.shape) != (n * 90, 32):
         raise CczError("heads_pack: h must be bf16 (n*90, 32) and operands bf16 (n, K)")
     with torch.cuda.device(h.device):
-        check(load().ccz_heads_pack(_ptr(h), n, _ptr(operands), int(operands.shape[1]), int(value_off), stream_ptr(h.device)),
-              "ccz_heads_pack")
+        if rows is None:
+            check(load().ccz_heads_pack(_ptr(h), n, _ptr(operands), int(operands.shape[1]), int(value_off), stream_ptr(h.device)),
+                  "ccz_heads_pack")
+        else:
+            if rows.dtype != torch.int32 or rows.numel() != n:
+                raise CczError("heads_pack: rows must be int32 (n,)")
+            check(load().ccz_heads_pack_rows(_ptr(h), n, _ptr(rows), _ptr(operands), int(operands.shape[1]), int(value_off),
+                                             stream_ptr(h.device)), "ccz_heads_pack_rows")
     return operands
+
+
+def leaf_unique(boards: torch.Tensor, rows: torch.Tensor, uniq: torch.Tensor, n_unique: torch.Tensor,
+                total: torch.Tensor | None = None) -> None:
+    """K12: the distinct positions (bytes 0..90) of ``boards`` (n,96) uint8.  Writes ``uniq`` (n,96) rows 0..U-1 with the
+    distinct records in order of first occurrence, ``rows`` int32 (n,) with each board's row in ``uniq``, ``n_unique``
+    int32 (1,) = U, and adds U to ``total`` (int64 (1,)) when given.  No host synchronisation."""
+    n = boards.shape[0]
+    if boards.dtype != torch.uint8 or boards.shape[1:] != (BOARD_BYTES,) or uniq.dtype != torch.uint8 or uniq.shape != boards.shape:
+        raise CczError("leaf_unique: boards and uniq must be uint8 (n,96)")
+    if rows.dtype != torch.int32 or rows.numel() != n:
+        raise CczError("leaf_unique: rows must be int32 (n,)")
+    _check_count(n_unique, boards.device)
+    if total is not None and (total.dtype != torch.int64 or total.numel() != 1):
+        raise CczError("leaf_unique: total must be int64 (1,)")
+    with torch.cuda.device(boards.device):
+        check(load().ccz_leaf_unique(_ptr(boards), n, _ptr(rows), _ptr(uniq), _ptr(n_unique), _ptr(total),
+                                     stream_ptr(boards.device)), "ccz_leaf_unique")
 
 
 def conv3x3_plan(n_boards: int, variant: int = 0, resident_clusters: int = 74) -> dict:

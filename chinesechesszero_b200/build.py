@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 OUT = os.path.join(CSRC, "libccz_b200.so")
 SOURCES = ["ccz_b200.cu"]
-HEADERS = ["ccz_rules.cuh", "ccz_movegen.cuh", "ccz_mcts.cuh", "ccz_replay.cuh", "ccz_conv.cuh", "ccz_stem.cuh", "ccz_heads.cuh", "../../include/ccz_b200.h"]
+HEADERS = ["ccz_rules.cuh", "ccz_movegen.cuh", "ccz_mcts.cuh", "ccz_replay.cuh", "ccz_conv.cuh", "ccz_stem.cuh", "ccz_heads.cuh", "ccz_dedup.cuh", "../../include/ccz_b200.h"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-lineinfo", "-O3", "-std=c++17",

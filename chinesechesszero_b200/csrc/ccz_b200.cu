@@ -16,6 +16,7 @@
 #include "ccz_conv.cuh"
 #include "ccz_stem.cuh"
 #include "ccz_heads.cuh"
+#include "ccz_dedup.cuh"
 
 #ifndef CCZ_CONV_DEFAULT_PAIRS
 #define CCZ_CONV_DEFAULT_PAIRS 1
@@ -449,55 +450,127 @@ int ccz_replay_pack(const uint8_t *d_hist_boards, const uint8_t *d_turn_plane, c
     return check_launch("replay_pi_kernel");
 }
 
-int ccz_conv3x3_c256(const void *d_x, const void *d_w, const float *d_bias, const void *d_skip, void *d_y, int n_boards,
-                     int variant, ccz_stream_t s) {
+}  // extern "C"
+
+namespace {
+
+// d_count == nullptr: n_boards boards.  Otherwise n_boards is the capacity the tensor maps are encoded for and the
+// kernel convolves min(*d_count, n_boards) boards.
+int conv3x3_c256_impl(const char *name, const void *d_x, const void *d_w, const float *d_bias, const void *d_skip, void *d_y,
+                      int n_boards, const int32_t *d_count, int variant, ccz_stream_t s) {
     namespace cv = ccz::conv;
-    if (n_boards < 0) return fail(-1, "ccz_conv3x3_c256: n_boards < 0");
+    std::string e_name(name);
+    auto bad = [&](int code, const char *what) { return fail(code, (e_name + ": " + what).c_str()); };
+    if (n_boards < 0) return bad(-1, "n_boards < 0");
     if (n_boards == 0) return 0;
-    if (!d_x || !d_w || !d_bias || !d_y) return fail(-1, "ccz_conv3x3_c256: NULL pointer");
-    if (d_y == d_x) return fail(-1, "ccz_conv3x3_c256: output must not alias the input (halo reads)");
-    if (variant < 0 || variant >= 128) return fail(-1, "ccz_conv3x3_c256: bad variant");
+    if (!d_x || !d_w || !d_bias || !d_y) return bad(-1, "NULL pointer");
+    if (d_y == d_x) return bad(-1, "output must not alias the input (halo reads)");
+    if (variant < 0 || variant >= 128) return bad(-1, "bad variant");
     // variant: 0 = default.  bits 0-1 CTA group (1 / 2), bit 2 = no tail split, bits 3-4 = traffic experiment
     // (skips loads, WRONG results), bits 5-6 = log2(CTA pairs per cluster sharing a weight stage)
     int cta_group = variant & 3;
     const int tail_split = !(variant & 4), dbg = (variant >> 3) & 3;
     int pairs = 1 << ((variant >> 5) & 3);
 #ifndef CCZ_CONV_EXPERIMENTS
-    if (dbg) return fail(-1, "ccz_conv3x3_c256: the load-skipping measurement variants need a -DCCZ_CONV_EXPERIMENTS build");
+    if (dbg) return bad(-1, "the load-skipping measurement variants need a -DCCZ_CONV_EXPERIMENTS build");
 #endif
     if (variant == 0) { cta_group = 2; pairs = CCZ_CONV_DEFAULT_PAIRS; }
     if (cta_group == 0) cta_group = 2;
     if (cta_group == 3 || pairs > 4 || (cta_group == 1 && pairs != 1))
-        return fail(-1, "ccz_conv3x3_c256: unsupported variant (cta_group 1|2, pairs 1|2|4, pairs > 1 needs cta_group 2)");
+        return bad(-1, "unsupported variant (cta_group 1|2, pairs 1|2|4, pairs > 1 needs cta_group 2)");
     if (((uintptr_t)d_x | (uintptr_t)d_w | (uintptr_t)d_y | (uintptr_t)d_skip) & 15)
-        return fail(-1, "ccz_conv3x3_c256: pointers must be 16-byte aligned");
+        return bad(-1, "pointers must be 16-byte aligned");
     static cv::Driver drv;
     if (const char *err = cv::driver_init(drv)) return fail(-3, err);
     const long long m = (long long)n_boards * cv::BOARD_HW;
     const int rows_per_tile = cv::BM * cta_group * pairs;
     const int n_tiles = (int)((m + rows_per_tile - 1) / rows_per_tile);
     CUtensorMap tx, tw, ts, ty;
-    if (!cv::encode_im2col(drv, &tx, d_x, n_boards)) return fail(-3, "ccz_conv3x3_c256: cuTensorMapEncodeIm2col(x) failed");
+    if (!cv::encode_im2col(drv, &tx, d_x, n_boards)) return bad(-3, "cuTensorMapEncodeIm2col(x) failed");
     if (!cv::encode_rows(drv, &tw, d_w, cv::BN, 9 * cv::C, (uint32_t)(cv::BN / cta_group / pairs)))
-        return fail(-3, "ccz_conv3x3_c256: cuTensorMapEncodeTiled(w) failed");
-    if (!cv::encode_rows(drv, &ty, d_y, (uint64_t)m, cv::C, cv::BM)) return fail(-3, "ccz_conv3x3_c256: cuTensorMapEncodeTiled(y) failed");
+        return bad(-3, "cuTensorMapEncodeTiled(w) failed");
+    if (!cv::encode_rows(drv, &ty, d_y, (uint64_t)m, cv::C, cv::BM)) return bad(-3, "cuTensorMapEncodeTiled(y) failed");
     if (d_skip) {
-        if (!cv::encode_rows(drv, &ts, d_skip, (uint64_t)m, cv::C, cv::BM))
-            return fail(-3, "ccz_conv3x3_c256: cuTensorMapEncodeTiled(skip) failed");
+        if (!cv::encode_rows(drv, &ts, d_skip, (uint64_t)m, cv::C, cv::BM)) return bad(-3, "cuTensorMapEncodeTiled(skip) failed");
     } else {
         ts = ty;
     }
     cudaError_t e;
-#define CCZ_CONV_LAUNCH(CG, PAIRS)                                                                                      \
-    (d_skip ? cv::launch_variant<CG, PAIRS, true>(tx, tw, ts, ty, d_bias, n_tiles, tail_split, dbg, s)     \
-            : cv::launch_variant<CG, PAIRS, false>(tx, tw, ts, ty, d_bias, n_tiles, tail_split, dbg, s))
+#define CCZ_CONV_LAUNCH_C(CG, PAIRS, CNT)                                                                                  \
+    (d_skip ? cv::launch_variant<CG, PAIRS, true, CNT>(tx, tw, ts, ty, d_bias, n_tiles, tail_split, dbg, d_count, n_boards, s) \
+            : cv::launch_variant<CG, PAIRS, false, CNT>(tx, tw, ts, ty, d_bias, n_tiles, tail_split, dbg, d_count, n_boards, s))
+#define CCZ_CONV_LAUNCH(CG, PAIRS) (d_count ? CCZ_CONV_LAUNCH_C(CG, PAIRS, true) : CCZ_CONV_LAUNCH_C(CG, PAIRS, false))
     if (cta_group == 1) e = CCZ_CONV_LAUNCH(1, 1);
     else if (pairs == 1) e = CCZ_CONV_LAUNCH(2, 1);
     else if (pairs == 2) e = CCZ_CONV_LAUNCH(2, 2);
     else e = CCZ_CONV_LAUNCH(2, 4);
 #undef CCZ_CONV_LAUNCH
+#undef CCZ_CONV_LAUNCH_C
     if (e != cudaSuccess) return fail(-2, "conv3x3_c256_kernel launch", e);
     return 0;
+}
+
+int stem_lookup_impl(const char *name, const uint8_t *d_boards, int n, const int32_t *d_count, const void *d_table,
+                     const float *d_bias_turn, void *d_y, ccz_stream_t s) {
+    namespace st = ccz::stem;
+    std::string e_name(name);
+    if (n < 0) return fail(-1, (e_name + ": n < 0").c_str());
+    if (n == 0) return 0;
+    if (!d_boards || !d_table || !d_bias_turn || !d_y) return fail(-1, (e_name + ": NULL pointer").c_str());
+    if (((uintptr_t)d_boards & 3) || (((uintptr_t)d_table | (uintptr_t)d_bias_turn | (uintptr_t)d_y) & 15))
+        return fail(-1, (e_name + ": pointers must be 16-byte aligned (boards 4-byte)").c_str());
+    static int n_sm_dev[64] = {0};
+    int dev = 0;
+    CCZ_CUDA(cudaGetDevice(&dev));
+    if (dev < 0 || dev >= 64) return fail(-1, (e_name + ": device index out of range").c_str());
+    int &n_sm = n_sm_dev[dev];
+    if (!n_sm) {
+        CCZ_CUDA(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev));
+        CCZ_CUDA(cudaFuncSetAttribute(st::stem_lookup_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, st::SMEM_BYTES));
+        CCZ_CUDA(cudaFuncSetAttribute(st::stem_lookup_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, st::SMEM_BYTES));
+    }
+    int blocks = 2 * n_sm; // two resident CTAs (92 KB of tables each) per SM
+    const int need = (n + st::WARPS - 1) / st::WARPS;
+    if (blocks > need) blocks = need;
+    const uint4 *tab = static_cast<const uint4 *>(d_table);
+    const float4 *bt = reinterpret_cast<const float4 *>(d_bias_turn);
+    uint4 *y = static_cast<uint4 *>(d_y);
+    if (d_count)
+        st::stem_lookup_kernel<true><<<blocks, st::WARPS * 32, st::SMEM_BYTES, s>>>(d_boards, n, tab, bt, y, d_count);
+    else
+        st::stem_lookup_kernel<false><<<blocks, st::WARPS * 32, st::SMEM_BYTES, s>>>(d_boards, n, tab, bt, y, nullptr);
+    return check_launch("stem_lookup_kernel");
+}
+
+int heads_pack_impl(const char *name, const void *d_h, int n, const int32_t *d_rows, void *d_operands, int row_elems, int value_off,
+                    ccz_stream_t s) {
+    namespace hd = ccz::heads;
+    std::string e_name(name);
+    if (n < 0) return fail(-1, (e_name + ": n < 0").c_str());
+    if (n == 0) return 0;
+    if (!d_h || !d_operands) return fail(-1, (e_name + ": NULL pointer").c_str());
+    if (((uintptr_t)d_h & 15) || ((uintptr_t)d_operands & 3) || ((uintptr_t)d_rows & 3))
+        return fail(-1, (e_name + ": h must be 16-byte, operands and rows 4-byte aligned").c_str());
+    if ((row_elems & 1) || (value_off & 1) || value_off < hd::N_POLICY * hd::HW || row_elems < value_off + hd::N_VALUE * hd::HW)
+        return fail(-1, (e_name + ": operand row must hold 1530 policy + 630 value elements at even offsets").c_str());
+    hd::heads_pack_kernel<<<n, hd::THREADS, 0, s>>>(static_cast<const uint4 *>(d_h), static_cast<uint32_t *>(d_operands), n,
+                                                  row_elems / 2, value_off / 2, d_rows);
+    return check_launch("heads_pack_kernel");
+}
+
+} // namespace
+
+extern "C" {
+
+int ccz_conv3x3_c256(const void *d_x, const void *d_w, const float *d_bias, const void *d_skip, void *d_y, int n_boards,
+                     int variant, ccz_stream_t s) {
+    return conv3x3_c256_impl("ccz_conv3x3_c256", d_x, d_w, d_bias, d_skip, d_y, n_boards, nullptr, variant, s);
+}
+
+int ccz_conv3x3_c256_count(const void *d_x, const void *d_w, const float *d_bias, const void *d_skip, void *d_y, int capacity,
+                           const int32_t *d_n_boards, int variant, ccz_stream_t s) {
+    if (!d_n_boards) return fail(-1, "ccz_conv3x3_c256_count: d_n_boards is NULL");
+    return conv3x3_c256_impl("ccz_conv3x3_c256_count", d_x, d_w, d_bias, d_skip, d_y, capacity, d_n_boards, variant, s);
 }
 
 int ccz_conv3x3_plan(int n_boards, int variant, int resident_clusters, int32_t *out) {
@@ -517,41 +590,46 @@ int ccz_conv3x3_plan(int n_boards, int variant, int resident_clusters, int32_t *
 }
 
 int ccz_stem_lookup(const uint8_t *d_boards, int n, const void *d_table, const float *d_bias_turn, void *d_y, ccz_stream_t s) {
-    namespace st = ccz::stem;
-    if (n < 0) return fail(-1, "ccz_stem_lookup: n < 0");
-    if (n == 0) return 0;
-    if (!d_boards || !d_table || !d_bias_turn || !d_y) return fail(-1, "ccz_stem_lookup: NULL pointer");
-    if (((uintptr_t)d_boards & 3) || (((uintptr_t)d_table | (uintptr_t)d_bias_turn | (uintptr_t)d_y) & 15))
-        return fail(-1, "ccz_stem_lookup: pointers must be 16-byte aligned (boards 4-byte)");
-    static int n_sm_dev[64] = {0};
-    int dev = 0;
-    CCZ_CUDA(cudaGetDevice(&dev));
-    if (dev < 0 || dev >= 64) return fail(-1, "ccz_stem_lookup: device index out of range");
-    int &n_sm = n_sm_dev[dev];
-    if (!n_sm) {
-        CCZ_CUDA(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev));
-        CCZ_CUDA(cudaFuncSetAttribute(st::stem_lookup_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, st::SMEM_BYTES));
-    }
-    int blocks = 2 * n_sm; // two resident CTAs (92 KB of tables each) per SM
-    const int need = (n + st::WARPS - 1) / st::WARPS;
-    if (blocks > need) blocks = need;
-    st::stem_lookup_kernel<<<blocks, st::WARPS * 32, st::SMEM_BYTES, s>>>(d_boards, n, static_cast<const uint4 *>(d_table),
-                                                                         reinterpret_cast<const float4 *>(d_bias_turn),
-                                                                         static_cast<uint4 *>(d_y));
-    return check_launch("stem_lookup_kernel");
+    return stem_lookup_impl("ccz_stem_lookup", d_boards, n, nullptr, d_table, d_bias_turn, d_y, s);
+}
+
+int ccz_stem_lookup_count(const uint8_t *d_boards, int capacity, const int32_t *d_n_boards, const void *d_table, const float *d_bias_turn,
+                          void *d_y, ccz_stream_t s) {
+    if (!d_n_boards) return fail(-1, "ccz_stem_lookup_count: d_n_boards is NULL");
+    return stem_lookup_impl("ccz_stem_lookup_count", d_boards, capacity, d_n_boards, d_table, d_bias_turn, d_y, s);
 }
 
 int ccz_heads_pack(const void *d_h, int n, void *d_operands, int row_elems, int value_off, ccz_stream_t s) {
-    namespace hd = ccz::heads;
-    if (n < 0) return fail(-1, "ccz_heads_pack: n < 0");
-    if (n == 0) return 0;
-    if (!d_h || !d_operands) return fail(-1, "ccz_heads_pack: NULL pointer");
-    if (((uintptr_t)d_h & 15) || ((uintptr_t)d_operands & 3)) return fail(-1, "ccz_heads_pack: h must be 16-byte, operands 4-byte aligned");
-    if ((row_elems & 1) || (value_off & 1) || value_off < hd::N_POLICY * hd::HW || row_elems < value_off + hd::N_VALUE * hd::HW)
-        return fail(-1, "ccz_heads_pack: operand row must hold 1530 policy + 630 value elements at even offsets");
-    hd::heads_pack_kernel<<<n, hd::THREADS, 0, s>>>(static_cast<const uint4 *>(d_h), static_cast<uint32_t *>(d_operands), n,
-                                                  row_elems / 2, value_off / 2);
-    return check_launch("heads_pack_kernel");
+    return heads_pack_impl("ccz_heads_pack", d_h, n, nullptr, d_operands, row_elems, value_off, s);
+}
+
+int ccz_heads_pack_rows(const void *d_h, int n, const int32_t *d_rows, void *d_operands, int row_elems, int value_off, ccz_stream_t s) {
+    if (!d_rows) return fail(-1, "ccz_heads_pack_rows: d_rows is NULL");
+    return heads_pack_impl("ccz_heads_pack_rows", d_h, n, d_rows, d_operands, row_elems, value_off, s);
+}
+
+int ccz_leaf_unique(const uint8_t *d_boards, int n, int32_t *d_rows, uint8_t *d_uniq_boards, int32_t *d_n_unique,
+                    unsigned long long *d_unique_total, ccz_stream_t s) {
+    namespace dd = ccz::dedup;
+    if (n < 0 || n > dd::MAX_BOARDS) return fail(-1, "ccz_leaf_unique: n must be 0..16384");
+    if (!d_n_unique) return fail(-1, "ccz_leaf_unique: d_n_unique is NULL");
+    if (n == 0) {
+        CCZ_CUDA(cudaMemsetAsync(d_n_unique, 0, sizeof(int32_t), s));
+        return 0;
+    }
+    if (!d_boards || !d_rows || !d_uniq_boards) return fail(-1, "ccz_leaf_unique: NULL pointer");
+    if (((uintptr_t)d_boards | (uintptr_t)d_uniq_boards) & 15) return fail(-1, "ccz_leaf_unique: boards must be 16-byte aligned");
+    if (d_uniq_boards == d_boards) return fail(-1, "ccz_leaf_unique: uniq_boards must not alias boards");
+    static bool attr_set[64] = {false};
+    int dev = 0;
+    CCZ_CUDA(cudaGetDevice(&dev));
+    if (dev < 0 || dev >= 64) return fail(-1, "ccz_leaf_unique: device index out of range");
+    if (!attr_set[dev]) {
+        CCZ_CUDA(cudaFuncSetAttribute(dd::leaf_unique_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, dd::smem_bytes(dd::MAX_BOARDS)));
+        attr_set[dev] = true;
+    }
+    dd::leaf_unique_kernel<<<1, dd::THREADS, dd::smem_bytes(n), s>>>(d_boards, n, d_rows, d_uniq_boards, d_n_unique, d_unique_total);
+    return check_launch("leaf_unique_kernel");
 }
 
 } // extern "C"

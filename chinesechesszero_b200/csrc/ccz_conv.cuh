@@ -294,14 +294,37 @@ __device__ __forceinline__ WorkItem work_item(int i, int n_full, int split_log2)
     return {n_full + (j >> split_log2), (j & ((1 << split_log2) - 1)) * n_w, n_w};
 }
 
+// Work plan of one launch: `n_tiles` cluster tiles over `clusters` resident clusters.  The tiles of the last, partial
+// round are sliced into 2 or 4 output-channel slices while every slice still gets its own cluster.
+struct Plan {
+    int n_items, n_full, split_log2, clusters;
+};
+__host__ __device__ inline Plan plan_items(int n_tiles, int clusters, bool tail_split) {
+    const int rem = n_tiles % clusters;
+    int split_log2 = 0;
+    if (tail_split && rem > 0) {
+        while (split_log2 < 2 && (rem << (split_log2 + 1)) <= clusters) ++split_log2;
+    }
+    Plan p;
+    p.split_log2 = split_log2;
+    p.n_full = split_log2 ? n_tiles - rem : n_tiles;
+    p.n_items = p.n_full + (split_log2 ? rem << split_log2 : 0);
+    p.clusters = clusters > p.n_items ? p.n_items : clusters;
+    return p;
+}
+
 // PAIRS > 1 (CG == 2 only): a cluster of PAIRS CTA pairs works on PAIRS consecutive tiles with the SAME weight
 // stage: each CTA fetches 1/PAIRS of its half of the weight tile and multicasts it to the CTAs of equal
 // parity, so weight traffic from L2 drops by PAIRS.  A stage is then free only when every pair has consumed it.
-template <int CG, int PAIRS, bool HAS_SKIP>
+//
+// DEV_COUNT: the board count is read from device memory (min(*d_count, count_cap), the tensor maps being encoded for
+// count_cap boards), and every CTA derives the plan from it as the host does; the grid is every resident cluster and
+// the clusters without an item only allocate / free TMEM and pass the cluster barriers.
+template <int CG, int PAIRS, bool HAS_SKIP, bool DEV_COUNT>
 __global__ void __launch_bounds__(THREADS, 1)
 conv3x3_c256_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUtensorMap tm_w,
                     const __grid_constant__ CUtensorMap tm_skip, const __grid_constant__ CUtensorMap tm_y, const float *__restrict__ bias,
-                    int n_items, int n_full, int split_log2, int dbg) {
+                    int n_items, int n_full, int split_log2, int dbg, const int32_t *__restrict__ d_count, int count_cap, int tail_split) {
     using K = Cfg<CG>;
     extern __shared__ uint8_t smem_raw[];
     const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -325,6 +348,13 @@ conv3x3_c256_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
     const uint32_t rank = CLUSTER > 1 ? cluster_ctarank() : 0u;
     const uint32_t prank = rank % CG, pair_id = rank / CG, lead_rank = rank - prank; // position in the pair / pair in the cluster
     const int cluster_id = blockIdx.x / CLUSTER, n_clusters = gridDim.x / CLUSTER;
+    if constexpr (DEV_COUNT) {
+        const int nb = min(max(*d_count, 0), count_cap), rows_per_tile = BM * CLUSTER;
+        const Plan pl = plan_items((nb * BOARD_HW + rows_per_tile - 1) / rows_per_tile, n_clusters, tail_split != 0);
+        n_items = pl.n_items;
+        n_full = pl.n_full;
+        split_log2 = pl.split_log2;
+    }
 
     if (warp == 0 && lane == 0) {
         tma_prefetch_desc(&tm_x);
@@ -556,29 +586,12 @@ inline bool encode_im2col(const Driver &d, CUtensorMap *m, const void *ptr, int 
                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-// Work plan of one launch: `n_tiles` cluster tiles over `clusters` resident clusters.  The tiles of the last, partial
-// round are sliced into 2 or 4 output-channel slices while every slice still gets its own cluster.
-struct Plan {
-    int n_items, n_full, split_log2, clusters;
-};
-inline Plan plan_items(int n_tiles, int clusters, bool tail_split) {
-    const int rem = n_tiles % clusters;
-    int split_log2 = 0;
-    if (tail_split && rem > 0) {
-        while (split_log2 < 2 && (rem << (split_log2 + 1)) <= clusters) ++split_log2;
-    }
-    Plan p;
-    p.split_log2 = split_log2;
-    p.n_full = split_log2 ? n_tiles - rem : n_tiles;
-    p.n_items = p.n_full + (split_log2 ? rem << split_log2 : 0);
-    p.clusters = clusters > p.n_items ? p.n_items : clusters;
-    return p;
-}
-
-template <int CG, int PAIRS, bool HAS_SKIP>
+// d_count == nullptr: `n_tiles` cluster tiles planned here.  Otherwise the kernel plans from min(*d_count, count_cap)
+// boards on the device and every resident cluster is launched.
+template <int CG, int PAIRS, bool HAS_SKIP, bool DEV_COUNT>
 inline cudaError_t launch_variant(const CUtensorMap &tx, const CUtensorMap &tw, const CUtensorMap &ts, const CUtensorMap &ty, const float *bias,
-                                  int n_tiles, int tail_split, int dbg, cudaStream_t stream) {
-    auto kern = conv3x3_c256_kernel<CG, PAIRS, HAS_SKIP>;
+                                  int n_tiles, int tail_split, int dbg, const int32_t *d_count, int count_cap, cudaStream_t stream) {
+    auto kern = conv3x3_c256_kernel<CG, PAIRS, HAS_SKIP, DEV_COUNT>;
     constexpr int CLUSTER = CG * PAIRS;
     // per device: resident clusters of this shape (GPC boundaries can strand SMs for CLUSTER > 2); function
     // attributes are per device too
@@ -611,9 +624,13 @@ inline cudaError_t launch_variant(const CUtensorMap &tx, const CUtensorMap &tw, 
         if (n < 1) return cudaErrorInvalidConfiguration;
         max_clusters = n < n_sm / CLUSTER ? n : n_sm / CLUSTER;
     }
+    if constexpr (DEV_COUNT) {
+        cfg.gridDim = dim3((unsigned)(max_clusters * CLUSTER));
+        return cudaLaunchKernelEx(&cfg, kern, tx, tw, ts, ty, bias, 0, 0, 0, dbg, d_count, count_cap, tail_split);
+    }
     const Plan pl = plan_items(n_tiles, max_clusters, tail_split != 0);
     cfg.gridDim = dim3((unsigned)(pl.clusters * CLUSTER));
-    return cudaLaunchKernelEx(&cfg, kern, tx, tw, ts, ty, bias, pl.n_items, pl.n_full, pl.split_log2, dbg);
+    return cudaLaunchKernelEx(&cfg, kern, tx, tw, ts, ty, bias, pl.n_items, pl.n_full, pl.split_log2, dbg, (const int32_t *)nullptr, 0, 0);
 }
 
 } // namespace conv

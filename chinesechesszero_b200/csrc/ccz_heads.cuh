@@ -6,7 +6,8 @@
 // contiguous 4-byte words into the K-padded rows the aligned cuBLAS kernels consume ([policy 1530 -> kp |
 // value 630 -> kv]; the pad columns are never written and stay zero).  Replaces three torch element-wise
 // launches (ReLU + two strided transposing copies, 2 x 48 us per 4096 boards) by one (HBM-bound: 5.8 KB in,
-// 4.3 KB out per board).
+// 4.3 KB out per board).  `rows` (may be NULL = identity): board b's operands come from h's board rows[b], so the
+// FC layers see G rows when the 1x1 GEMM ran on K12's compacted distinct leaves.
 #pragma once
 #include <cuda_bf16.h>
 #include <stdint.h>
@@ -18,11 +19,11 @@ constexpr int HW = 90, CH = 32, N_POLICY = 17, N_VALUE = 7, THREADS = 128;
 
 __global__ void __launch_bounds__(THREADS)
 heads_pack_kernel(const uint4 *__restrict__ h /*[n*90*32 bf16]*/, uint32_t *__restrict__ out /*[n][row_words]*/, int n,
-                  int row_words, int value_word_off) {
+                  int row_words, int value_word_off, const int32_t *__restrict__ rows) {
     __shared__ __align__(16) uint16_t s_t[HW][CH + 2]; // +2 halfwords: the column reads below hit distinct banks
     const int b = blockIdx.x;
     if (b >= n) return;
-    const uint4 *src = h + (size_t)b * (HW * CH * 2 / 16);
+    const uint4 *src = h + (size_t)(rows ? rows[b] : b) * (HW * CH * 2 / 16);
     for (int i = threadIdx.x; i < HW * CH * 2 / 16; i += THREADS) {
         const uint4 v = src[i];
         const int row = i >> 2, col = (i & 3) * 8; // 4 vectors of 8 channels per pixel row

@@ -13,7 +13,8 @@
 //
 // No planes are read (21 KB / position saved), no channel padding, no layout copy: the kernel is bound by
 // the 46 KB / board NHWC bf16 output it writes.  One warp per board, lane = 8 output channels; tables
-// (92 KB) staged in shared memory once per persistent CTA.
+// (92 KB) staged in shared memory once per persistent CTA.  DEV_COUNT: the board count is min(*d_count, n), read
+// on the device (K12's number of distinct leaves); warps past it exit.
 #pragma once
 
 #include <cuda_bf16.h>
@@ -40,9 +41,11 @@ __device__ __forceinline__ void add_row(float (&acc)[8], const uint4 t) {
     }
 }
 
+template <bool DEV_COUNT>
 __global__ void __launch_bounds__(WARPS * 32, 2)
 stem_lookup_kernel(const uint8_t *__restrict__ boards, int n, const uint4 *__restrict__ table, const float4 *__restrict__ bias_turn,
-                   uint4 *__restrict__ y) {
+                   uint4 *__restrict__ y, const int32_t *__restrict__ d_count) {
+    if constexpr (DEV_COUNT) n = min(*d_count, n);
     extern __shared__ __align__(16) uint8_t smem[];
     uint4 *tab_s = reinterpret_cast<uint4 *>(smem);
     float4 *bt_s = reinterpret_cast<float4 *>(smem + TABLE_ELEMS * 2);

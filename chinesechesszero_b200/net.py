@@ -119,6 +119,11 @@ class BatchedEvaluator:
 
     ``__call__(planes, leaf_boards) -> (logits fp32 (G,2086), POLICY_LOGITS, values fp32 (G,))``
     which is the evaluator protocol of :class:`search.LockstepSearch`.
+
+    ``dedup`` (default on): when the stem runs from the board records (K10) and the whole tower on K9, K12 first
+    compacts the leaf batch to its U distinct positions; K10 and K9 then run on U boards (the count stays on the
+    device), the 1x1 heads GEMM on the compacted buffer, and K11 packs each game's FC operands from its position's
+    row.  Results are bit-identical to ``dedup=False``: every board's forward output is independent of its row.
     """
 
     #: which kernel runs the 3x3 tower convolutions:
@@ -130,7 +135,7 @@ class BatchedEvaluator:
     CONV_IMPLS = ("k9", "k9_skip", "cudnn", "torch")
 
     def __init__(self, net: Net, device="cuda", dtype=torch.bfloat16, fused_epilogue: bool = True,
-                 conv_impl: str | None = None, chunk: int | None = None):
+                 conv_impl: str | None = None, chunk: int | None = None, dedup: bool = True):
         self.device = torch.device(device)
         self.dtype = dtype
         # leaves per sub-batch (0 = whole batch at once): sub-batches whose activations fit the 126 MB L2
@@ -145,7 +150,12 @@ class BatchedEvaluator:
             conv_impl = "cudnn"  # K9 is specialised for the 256-channel bf16 tower of the reference net
         self.conv_impl = conv_impl
         self.fused = conv_impl != "torch"
+        self.dedup = bool(dedup)
         self.n_evals = 0
+        # boards the forward actually ran on: host part (calls without dedup) + device accumulator of K12's counts
+        self._n_unique_host = 0
+        self._unique_total = torch.zeros(1, dtype=torch.int64, device=self.device) if self.device.type == "cuda" else None
+        self._dedup_buf: dict = {}
         self.use_heads_pack = os.environ.get("CCZ_HEADS_PACK", "1") != "0"  # K11; "0" = the torch copies (A/B measurements)
         # measurement hook (bench.py): when a list, every K9 launch of the next forwards is bracketed by CUDA
         # events on the launching stream and the (with_skip, start, end) triples are appended to it
@@ -218,28 +228,28 @@ class BatchedEvaluator:
         self.value_fc2 = (keep("vfc2.w", net.value_fc2.weight.detach().to(dev, torch.float32).clone()),
                           keep("vfc2.b", net.value_fc2.bias.detach().to(dev, torch.float32).clone()))
 
-    def _k9(self, x, w, b32, skip, out):
+    def _k9(self, x, w, b32, skip, out, count=None):
         if self.conv_events is None:
-            return _lib.conv3x3_c256(x, w, b32, skip=skip, out=out)
+            return _lib.conv3x3_c256(x, w, b32, skip=skip, out=out, count=count)
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        y = _lib.conv3x3_c256(x, w, b32, skip=skip, out=out)
+        y = _lib.conv3x3_c256(x, w, b32, skip=skip, out=out, count=count)
         e1.record()
         self.conv_events.append((skip is not None, e0, e1))
         return y
 
-    def _conv_relu(self, x, wb, k9=False):
+    def _conv_relu(self, x, wb, k9=False, count=None):
         w, b, b32 = wb
         if k9:
-            return self._k9(x, w, b32, None, None)
+            return self._k9(x, w, b32, None, None, count)
         if self.fused:
             return torch.cudnn_convolution_relu(x, w, b, (1, 1), (1, 1), (1, 1), 1)
         return F.relu_(F.conv2d(x, w, b, padding=1))
 
-    def _conv_add_relu(self, x, wb, skip, k9=False):
+    def _conv_add_relu(self, x, wb, skip, k9=False, count=None):
         w, b, b32 = wb
         if k9:  # the block's output overwrites its input (each tile reads its skip rows before storing them)
-            return self._k9(x, w, b32, skip, skip)
+            return self._k9(x, w, b32, skip, skip, count)
         if self.fused:
             return torch.cudnn_convolution_add_relu(x, w, skip, 1.0, b, (1, 1), (1, 1), (1, 1), 1)
         return F.relu_(F.conv2d(x, w, b, padding=1).add_(skip))
@@ -262,18 +272,45 @@ class BatchedEvaluator:
             return torch.cat([p[0] for p in parts]), torch.cat([p[1] for p in parts])
         return self._forward(None if use_boards else planes, boards if use_boards else None)
 
+    @property
+    def n_unique(self) -> int:
+        """Boards the forwards so far ran on (distinct leaves where dedup applied); reading it synchronises."""
+        dev = int(self._unique_total.item()) if self._unique_total is not None else 0
+        return self._n_unique_host + dev
+
+    def _dedup_buffers(self, g: int):
+        """(rows int32 (g,), uniq boards uint8 (g,96), n_unique int32 (1,)) kept per batch size: fixed addresses for
+        captured graphs."""
+        buf = self._dedup_buf.get(g)
+        if buf is None:
+            z = dict(device=self.device)
+            buf = self._dedup_buf[g] = (torch.zeros(g, dtype=torch.int32, **z), torch.zeros((g, _lib.BOARD_BYTES), dtype=torch.uint8, **z),
+                                        torch.zeros(1, dtype=torch.int32, **z))
+            if len(self._dedup_buf) > 8:
+                self._dedup_buf.pop(next(iter(self._dedup_buf)))
+        return buf
+
     def _forward(self, planes, boards=None):
+        row_map = count = None
         if boards is not None:
             g = boards.shape[0]
-            x = _lib.stem_lookup(boards, *self.stem_lookup)
+            if self.dedup and self.conv_impl == "k9" and g <= _lib.DEDUP_MAX_BOARDS:
+                # K12: forward the distinct positions only (rows 0..U-1); rows >= U of every activation are don't-care
+                row_map, uniq, count = self._dedup_buffers(g)
+                _lib.leaf_unique(boards, row_map, uniq, count, self._unique_total)
+                boards = uniq
+            else:
+                self._n_unique_host += g
+            x = _lib.stem_lookup(boards, *self.stem_lookup, count=count)
         else:
             g = planes.shape[0]
             x = planes.view(g, PLAYS * PIECES, 10, 9).contiguous(memory_format=torch.channels_last)
             x = self._conv_relu(x, self.stem)
+            self._n_unique_host += g
         k9_plain, k9_skip = self.conv_impl == "k9", self.conv_impl in ("k9", "k9_skip")
         for c1, c2 in self.blocks:
-            y = self._conv_relu(x, c1, k9_plain)
-            x = self._conv_add_relu(y, c2, x, k9_skip)
+            y = self._conv_relu(x, c1, k9_plain, count)
+            x = self._conv_add_relu(y, c2, x, k9_skip, count)
         if self.device.type == "cuda":
             # 1x1 heads = a GEMM over the (g*90, C) NHWC pixel rows (a view of the channels_last activations)
             rows = x.permute(0, 2, 3, 1).reshape(g * 90, x.shape[1])
@@ -284,10 +321,13 @@ class BatchedEvaluator:
                 if len(self._head_buf) > 8:
                     self._head_buf.pop(next(iter(self._head_buf)))
             if self.dtype == torch.bfloat16 and self.use_heads_pack:
-                # K11: ReLU + NHWC -> NCHW flatten order (channel-major within a board, net.py:97) in one launch
-                _lib.heads_pack(h, buf, self._kp)
+                # K11: ReLU + NHWC -> NCHW flatten order (channel-major within a board, net.py:97) in one launch;
+                # with dedup, game b's operands come from its position's compacted row row_map[b]
+                _lib.heads_pack(h, buf, self._kp, rows=row_map)
             else:
                 h = F.relu_(h).view(g, 90, 32)
+                if row_map is not None:
+                    h = h.index_select(0, row_map)
                 buf[:, :PLAYS * 90].view(g, PLAYS, 90).copy_(h[:, :, :PLAYS].transpose(1, 2))
                 buf[:, self._kp:self._kp + PIECES * 90].view(g, PIECES, 90).copy_(h[:, :, PLAYS:PLAYS + PIECES].transpose(1, 2))
             logits = F.linear(buf[:, :self._kp], self._fc_pad[0])[:, :N_ACTIONS].float() + self.policy_fc[1]

@@ -237,6 +237,14 @@ int ccz_replay_pack(const uint8_t *d_hist_boards /*[n,8,96]: history slots, most
 int ccz_conv3x3_c256(const void *d_x, const void *d_w, const float *d_bias, const void *d_skip, void *d_y,
                      int n_boards, int variant, ccz_stream_t s);
 
+/* K9 over a board count that lives on the device: the buffers hold `capacity` boards (the tensor maps are encoded
+ * for it) and the kernel convolves the first min(*d_n_boards, capacity) of them, planning its work items on the
+ * device exactly as ccz_conv3x3_plan does for that count.  Every resident cluster is launched; clusters without an
+ * item exit.  Output rows past the count (up to the end of the last tile) hold unspecified values.  Capture-safe: no
+ * host synchronisation.  Each board's output is bit-identical to ccz_conv3x3_c256 over the same boards. */
+int ccz_conv3x3_c256_count(const void *d_x, const void *d_w, const float *d_bias, const void *d_skip, void *d_y,
+                           int capacity, const int32_t *d_n_boards, int variant, ccz_stream_t s);
+
 /* Host-only: the work plan ccz_conv3x3_c256 would launch for n_boards on a device with `resident_clusters`
  * co-resident clusters of the variant's shape (74 CTA pairs on a B200).  out[6] = {pixel rows per cluster tile,
  * cluster tiles, work items, whole-tile items, log2 of the channel slices of the last partial round, clusters
@@ -256,12 +264,31 @@ int ccz_conv3x3_plan(int n_boards, int variant, int resident_clusters, int32_t *
 int ccz_stem_lookup(const uint8_t *d_boards, int n, const void *d_table, const float *d_bias_turn, void *d_y,
                     ccz_stream_t s);
 
+/* K10 over the first min(*d_n_boards, capacity) boards of d_boards (the count read on the device); output rows
+ * past the count are not written. */
+int ccz_stem_lookup_count(const uint8_t *d_boards, int capacity, const int32_t *d_n_boards, const void *d_table,
+                          const float *d_bias_turn, void *d_y, ccz_stream_t s);
+
 /* K11: ReLU + NHWC -> channel-major packing between the fused 1x1 head convolutions and the FC layers of
  * Net.forward (net.py:94-107).  d_h: bf16 [n*90][32] head-convolution outputs per pixel row (channels 0..16 policy,
  * 17..23 value, bias added, before the ReLU).  d_operands: bf16 [n][row_elems]; row b receives
  * relu(policy) as x.view(-1, 17*90) (net.py:97) at element 0 and relu(value) as x.view(-1, 7*90) (net.py:104) at element
  * value_off; other elements of the row (GEMM K padding) are left untouched. */
 int ccz_heads_pack(const void *d_h, int n, void *d_operands, int row_elems, int value_off, ccz_stream_t s);
+
+/* K11 with a row map: operand row b is packed from board d_rows[b] of d_h (each d_rows[b] must be a board of d_h).
+ * With ccz_leaf_unique's rows this expands the heads of the distinct leaves back to one operand row per game. */
+int ccz_heads_pack_rows(const void *d_h, int n, const int32_t *d_rows, void *d_operands, int row_elems, int value_off,
+                        ccz_stream_t s);
+
+/* K12: the distinct positions of a leaf batch.  Identity is bytes 0..90 of the record (squares + side to move, all
+ * the search-time net input depends on; boards that differ only in the clock or repetition bytes are one position).
+ * d_boards [n,96] -> d_uniq_boards [n,96]: the distinct records in rows 0..U-1 in order of first occurrence (lowest
+ * game index), rows >= U untouched; d_rows[g] = the row of game g's position; *d_n_unique = U; d_unique_total
+ * (may be NULL) += U.  One launch, no host synchronisation, no allocation (capture-safe); n <= 16384; both board
+ * arrays 16-byte aligned and distinct. */
+int ccz_leaf_unique(const uint8_t *d_boards, int n, int32_t *d_rows, uint8_t *d_uniq_boards, int32_t *d_n_unique,
+                    unsigned long long *d_unique_total, ccz_stream_t s);
 
 #ifdef __cplusplus
 }

@@ -12,7 +12,7 @@ from chinesechesszero_b200.net import BatchedEvaluator, Net
 
 G = int(os.environ.get("CCZ_G", "4096"))
 torch.manual_seed(0)
-ev = BatchedEvaluator(Net().cuda().eval())
+ev = BatchedEvaluator(Net().cuda().eval(), dedup=False)  # G copies of one board: time G boards, not one
 boards = _lib.boards_start(G)
 res = {"k11": [], "torch": []}
 for rnd in range(4):

@@ -16,7 +16,7 @@ USE_BOARDS = bool(os.environ.get("BOARDS"))
 ref = None
 for impl in impls:
     impl, _, chunk = impl.partition(":")
-    ev = BatchedEvaluator(net, conv_impl=impl, chunk=int(chunk or 0))
+    ev = BatchedEvaluator(net, conv_impl=impl, chunk=int(chunk or 0), dedup=False)  # G copies of one board
     for _ in range(3):
         logits, v = ev.forward(planes, boards if USE_BOARDS else None)
     torch.cuda.synchronize()

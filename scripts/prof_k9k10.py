@@ -7,7 +7,7 @@ from chinesechesszero_b200.net import Net, BatchedEvaluator
 
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 4096
 torch.manual_seed(0)
-ev = BatchedEvaluator(Net(resblocks_num=1).cuda().eval(), conv_impl="k9")
+ev = BatchedEvaluator(Net(resblocks_num=1).cuda().eval(), conv_impl="k9", dedup=False)
 boards = torch.empty(n, 96, dtype=torch.uint8, device="cuda")
 _lib.check(_lib.load().ccz_boards_start(boards.data_ptr(), n, _lib.stream_ptr()), "boards_start")
 for _ in range(3):
