@@ -39,6 +39,7 @@ EXPORTS = (
     "ccz_mcts_reserve", "ccz_mcts_migrate", "ccz_mcts_select",
     "ccz_mcts_expand_backup", "ccz_mcts_root_visits", "ccz_mcts_advance", "ccz_replay_pack", "ccz_conv3x3_c256", "ccz_conv3x3_plan", "ccz_stem_lookup",
     "ccz_heads_pack", "ccz_conv3x3_c256_count", "ccz_stem_lookup_count", "ccz_heads_pack_rows", "ccz_leaf_unique",
+    "ccz_conv3x3_c256_e4m3", "ccz_stem_lookup_e4m3",
 )
 
 
@@ -127,6 +128,8 @@ def load() -> ctypes.CDLL:
     lib.ccz_stem_lookup_count.argtypes = [vp, i32, vp, vp, vp, vp, vp]
     lib.ccz_heads_pack_rows.argtypes = [vp, i32, vp, vp, i32, i32, vp]
     lib.ccz_leaf_unique.argtypes = [vp, i32, vp, vp, vp, vp, vp]
+    lib.ccz_conv3x3_c256_e4m3.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, i32, vp, vp]
+    lib.ccz_stem_lookup_e4m3.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp, vp]
     for name in EXPORTS:
         if name not in ("ccz_last_error",):
             getattr(lib, name).restype = i32
@@ -441,6 +444,103 @@ def conv3x3_c256(x: torch.Tensor, w: torch.Tensor, bias: torch.Tensor, skip: tor
     return out
 
 
+E4M3 = torch.float8_e4m3fn
+E4M3_MAX = 448.0
+
+
+def _check_nhwc(name: str, what: str, t: torch.Tensor, dtype, n: int | None = None) -> None:
+    cl = torch.channels_last
+    if t.dtype != dtype or t.dim() != 4 or tuple(t.shape[1:]) != (256, 10, 9) or (n is not None and t.shape[0] != n) \
+            or not t.is_contiguous(memory_format=cl) or not t.is_cuda:
+        raise CczError(f"{name}: {what} must be a {dtype} (n,256,10,9) channels_last device tensor")
+
+
+def _check_scalar(name: str, what: str, t: torch.Tensor, dev) -> None:
+    if t.dtype != torch.float32 or t.numel() != 1 or t.device != dev:
+        raise CczError(f"{name}: {what} must be a one-element float32 tensor on the same device")
+
+
+def conv3x3_c256_e4m3(xq: torch.Tensor, wq: torch.Tensor, dequant: torch.Tensor, bias: torch.Tensor, skip: torch.Tensor | None = None,
+                      out: torch.Tensor | None = None, out_q: torch.Tensor | None = None, inv_s_out: torch.Tensor | None = None,
+                      y: bool = True, count: torch.Tensor | None = None):
+    """K9 with e4m3 operands: ``f = relu(conv3x3_pad1(xq, wq) * dequant + bias [+ skip])`` on the tcgen05 tensor cores.
+
+    ``xq`` e4m3 ``(n,256,10,9)`` channels_last; ``wq`` e4m3 ``(256,256,3,3)`` channels_last; ``dequant`` / ``bias`` fp32
+    (256,) (dequant[co] = input scale x weight scale of co); ``skip`` bf16 like ``xq`` (may be ``out``).  Outputs: the bf16
+    ``out`` = bf16(f) when ``y`` (allocated unless given) and, when ``inv_s_out`` (fp32 (1,) device tensor) is given, the
+    e4m3 ``out_q`` = satfinite(f * inv_s_out) (allocated unless given).  ``count`` as in :func:`conv3x3_c256`.
+    Returns ``(out or None, out_q or None)``."""
+    name = "conv3x3_c256_e4m3"
+    _check_nhwc(name, "xq", xq, E4M3)
+    n = xq.shape[0]
+    if wq.dtype != E4M3 or tuple(wq.shape) != (256, 256, 3, 3) or not wq.is_contiguous(memory_format=torch.channels_last):
+        raise CczError(f"{name}: wq must be float8_e4m3fn (256,256,3,3) channels_last")
+    for what, t in (("dequant", dequant), ("bias", bias)):
+        if t.dtype != torch.float32 or t.numel() != 256 or not t.is_contiguous() or t.device != xq.device:
+            raise CczError(f"{name}: {what} must be a contiguous float32 (256,) tensor on the device of xq")
+    if wq.device != xq.device:
+        raise CczError(f"{name}: wq must be on the device of xq")
+    if skip is not None:
+        _check_nhwc(name, "skip", skip, torch.bfloat16, n)
+    if y:
+        if out is None:
+            out = torch.empty((n, 256, 10, 9), dtype=torch.bfloat16, device=xq.device).contiguous(memory_format=torch.channels_last)
+        _check_nhwc(name, "out", out, torch.bfloat16, n)
+    else:
+        out = None
+    if inv_s_out is not None:
+        _check_scalar(name, "inv_s_out", inv_s_out, xq.device)
+        if out_q is None:
+            out_q = torch.empty((n, 256, 10, 9), dtype=E4M3, device=xq.device).contiguous(memory_format=torch.channels_last)
+        _check_nhwc(name, "out_q", out_q, E4M3, n)
+    elif out_q is not None:
+        raise CczError(f"{name}: out_q needs inv_s_out")
+    if count is not None:
+        _check_count(count, xq.device)
+    with torch.cuda.device(xq.device):
+        check(load().ccz_conv3x3_c256_e4m3(xq.data_ptr(), wq.data_ptr(), dequant.data_ptr(), bias.data_ptr(), _ptr_or_none(skip),
+                                           _ptr_or_none(out), _ptr_or_none(out_q), _ptr_or_none(inv_s_out), n, _ptr_or_none(count),
+                                           stream_ptr(xq.device)), "ccz_conv3x3_c256_e4m3")
+    return out, out_q
+
+
+def _ptr_or_none(t: torch.Tensor | None) -> int | None:
+    return None if t is None else t.data_ptr()
+
+
+def stem_lookup_e4m3(boards: torch.Tensor, table: torch.Tensor, bias_turn: torch.Tensor, inv_s_out: torch.Tensor,
+                     out: torch.Tensor | None = None, out_q: torch.Tensor | None = None, count: torch.Tensor | None = None):
+    """K10 with an e4m3 copy of its output: ``(y bf16, yq e4m3)``, both ``(n,256,10,9)`` channels_last, with
+    ``yq = satfinite(y * inv_s_out)`` (fp32 (1,) device tensor).  Other arguments as :func:`stem_lookup`."""
+    name = "stem_lookup_e4m3"
+    n = boards.shape[0]
+    _check_scalar(name, "inv_s_out", inv_s_out, boards.device)
+    if out_q is None:
+        out_q = torch.empty((n, 256, 10, 9), dtype=E4M3, device=boards.device).contiguous(memory_format=torch.channels_last)
+    _check_nhwc(name, "out_q", out_q, E4M3, n)
+    out = _stem_args(name, boards, table, bias_turn, out)
+    if count is not None:
+        _check_count(count, boards.device)
+    with torch.cuda.device(boards.device):
+        check(load().ccz_stem_lookup_e4m3(_ptr(boards), n, _ptr_or_none(count), _ptr(table), _ptr(bias_turn), out.data_ptr(),
+                                          out_q.data_ptr(), inv_s_out.data_ptr(), stream_ptr(boards.device)), "ccz_stem_lookup_e4m3")
+    return out, out_q
+
+
+def _stem_args(name, boards, table, bias_turn, out):
+    n = boards.shape[0]
+    if boards.dtype != torch.uint8 or boards.shape[1:] != (BOARD_BYTES,):
+        raise CczError(f"{name}: boards must be uint8 (n,96)")
+    if table.dtype != torch.bfloat16 or tuple(table.shape) != (9, 16, 256) or bias_turn.dtype != torch.float32 \
+            or tuple(bias_turn.shape) != (2, 9, 256):
+        raise CczError(f"{name}: table must be bf16 (9,16,256) and bias_turn fp32 (2,9,256)")
+    if out is None:
+        out = torch.empty((n, 256, 10, 9), dtype=torch.bfloat16, device=boards.device).contiguous(memory_format=torch.channels_last)
+    elif tuple(out.shape) != (n, 256, 10, 9) or out.dtype != torch.bfloat16 or not out.is_contiguous(memory_format=torch.channels_last):
+        raise CczError(f"{name}: out must be bf16 (n,256,10,9) channels_last")
+    return out
+
+
 def stem_lookup(boards: torch.Tensor, table: torch.Tensor, bias_turn: torch.Tensor, out: torch.Tensor | None = None,
                 count: torch.Tensor | None = None) -> torch.Tensor:
     """K10: stem conv + BN + ReLU of search-time inputs straight from ``boards`` (n,96) uint8 ->
@@ -448,15 +548,7 @@ def stem_lookup(boards: torch.Tensor, table: torch.Tensor, bias_turn: torch.Tens
     (built by ``net.stem_tables``).  ``count``: int32 (1,) device tensor -- only the first ``count`` boards
     are evaluated (``ccz_stem_lookup_count``), later output rows are not written."""
     n = boards.shape[0]
-    if boards.dtype != torch.uint8 or boards.shape[1:] != (BOARD_BYTES,):
-        raise CczError("stem_lookup: boards must be uint8 (n,96)")
-    if table.dtype != torch.bfloat16 or tuple(table.shape) != (9, 16, 256) or bias_turn.dtype != torch.float32 \
-            or tuple(bias_turn.shape) != (2, 9, 256):
-        raise CczError("stem_lookup: table must be bf16 (9,16,256) and bias_turn fp32 (2,9,256)")
-    if out is None:
-        out = torch.empty((n, 256, 10, 9), dtype=torch.bfloat16, device=boards.device).contiguous(memory_format=torch.channels_last)
-    elif tuple(out.shape) != (n, 256, 10, 9) or out.dtype != torch.bfloat16 or not out.is_contiguous(memory_format=torch.channels_last):
-        raise CczError("stem_lookup: out must be bf16 (n,256,10,9) channels_last")
+    out = _stem_args("stem_lookup", boards, table, bias_turn, out)
     with torch.cuda.device(boards.device):
         if count is None:
             check(load().ccz_stem_lookup(_ptr(boards), n, _ptr(table), _ptr(bias_turn), out.data_ptr(), stream_ptr(boards.device)),

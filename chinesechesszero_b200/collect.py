@@ -29,7 +29,7 @@ class CollectPipeline:
     def __init__(self, init_model=None, n_games=4096, n_playout=PLAYOUT, c_puct=C_PUCT, data_dir=DATA_DIR,
                  states_mode="reference", seed=0, node_cap=None, max_game_moves=None, net_kwargs=None,
                  write_h5=True, write_npy=True, rank=0, world=1, gzip_level=4, h5_flush_every=None,
-                 async_writer=True, evaluator=None):
+                 async_writer=True, evaluator=None, precision="bf16"):
         self.temp = 1.0
         self.n_playout = n_playout
         self.c_puct = c_puct
@@ -39,6 +39,7 @@ class CollectPipeline:
         self.policy_value_net = None
         self.engine = None
         self._evaluator = evaluator  # a ready device evaluator instead of loading a model (benchmarks, tests)
+        self.precision = precision  # of the evaluator built over the loaded model: "bf16" or "fp8" (BatchedEvaluator)
         self.rank, self.world = int(rank), int(world)
         self.data_dir = data_dir if self.world == 1 else os.path.join(data_dir, f"rank{self.rank}")
         self.data_path = os.path.join(self.data_dir, "data.h5")
@@ -73,7 +74,7 @@ class CollectPipeline:
                     self.policy_value_net = PolicyValueNet(model=model_path, **self.net_kwargs)
                 except Exception:
                     self.policy_value_net = PolicyValueNet(**self.net_kwargs)
-                evaluator = self.policy_value_net.evaluator()
+                evaluator = self.policy_value_net.evaluator(precision=self.precision)
             self.engine = SelfPlayEngine(evaluator, n_games=self.n_games, n_playout=self.n_playout,
                                          c_puct=self.c_puct, temp=self.temp, seed=self.seed,
                                          node_cap=self.node_cap, max_game_moves=self.max_game_moves)

@@ -510,14 +510,63 @@ int conv3x3_c256_impl(const char *name, const void *d_x, const void *d_w, const 
     return 0;
 }
 
+// e4m3 tower convolution: always CTA pairs (cta_group::2), one pair per cluster, tail split on.
+int conv3x3_c256_e4m3_impl(const void *d_xq, const void *d_wq, const float *d_dequant, const float *d_bias, const void *d_skip, void *d_y,
+                           void *d_yq, const float *d_inv_s_out, int n_boards, const int32_t *d_count, ccz_stream_t s) {
+    namespace cv = ccz::conv;
+    using E = __nv_fp8_e4m3;
+    auto bad = [&](int code, const char *what) { return fail(code, (std::string("ccz_conv3x3_c256_e4m3: ") + what).c_str()); };
+    if (n_boards < 0) return bad(-1, "capacity < 0");
+    if (n_boards == 0) return 0;
+    if (!d_xq || !d_wq || !d_dequant || !d_bias) return bad(-1, "NULL pointer");
+    if (!d_y && !d_yq) return bad(-1, "no output (d_y and d_yq are both NULL)");
+    if (d_yq && !d_inv_s_out) return bad(-1, "d_yq needs d_inv_s_out");
+    if (d_y == d_xq || d_yq == d_xq) return bad(-1, "outputs must not alias the input (halo reads)");
+    if (d_yq && (d_yq == d_y || d_yq == d_skip)) return bad(-1, "d_yq must not alias d_y or d_skip");
+    if (((uintptr_t)d_xq | (uintptr_t)d_wq | (uintptr_t)d_y | (uintptr_t)d_yq | (uintptr_t)d_skip | (uintptr_t)d_dequant |
+         (uintptr_t)d_bias) & 15)
+        return bad(-1, "pointers must be 16-byte aligned");
+    static cv::Driver drv;
+    if (const char *err = cv::driver_init(drv)) return fail(-3, err);
+    const long long m = (long long)n_boards * cv::BOARD_HW;
+    const int rows_per_tile = cv::BM * 2;
+    const int n_tiles = (int)((m + rows_per_tile - 1) / rows_per_tile);
+    CUtensorMap tx, tw, ts, ty;
+    if (!cv::encode_im2col(drv, &tx, d_xq, n_boards, true)) return bad(-3, "cuTensorMapEncodeIm2col(xq) failed");
+    if (!cv::encode_rows(drv, &tw, d_wq, cv::BN, 9 * cv::C, (uint32_t)(cv::BN / 2), true)) return bad(-3, "cuTensorMapEncodeTiled(wq) failed");
+    // without a bf16 output the y map is encoded over the skip (or the input) and never stored through
+    const void *y_map = d_y ? d_y : (d_skip ? d_skip : d_xq);
+    if (!cv::encode_rows(drv, &ty, y_map, (uint64_t)m, cv::C, cv::BM, !d_y && !d_skip)) return bad(-3, "cuTensorMapEncodeTiled(y) failed");
+    if (d_skip) {
+        if (!cv::encode_rows(drv, &ts, d_skip, (uint64_t)m, cv::C, cv::BM)) return bad(-3, "cuTensorMapEncodeTiled(skip) failed");
+    } else {
+        ts = ty;
+    }
+    cv::QOut<E> qo;
+    qo.dequant = d_dequant;
+    qo.yq = static_cast<uint8_t *>(d_yq);
+    qo.inv_s_out = d_inv_s_out;
+    qo.rows = m;
+    qo.out_y = d_y != nullptr;
+    cudaError_t e;
+    if (d_count)
+        e = d_skip ? cv::launch_variant<2, 1, true, true, E>(tx, tw, ts, ty, d_bias, n_tiles, 1, 0, d_count, n_boards, s, qo)
+                   : cv::launch_variant<2, 1, false, true, E>(tx, tw, ts, ty, d_bias, n_tiles, 1, 0, d_count, n_boards, s, qo);
+    else
+        e = d_skip ? cv::launch_variant<2, 1, true, false, E>(tx, tw, ts, ty, d_bias, n_tiles, 1, 0, nullptr, n_boards, s, qo)
+                   : cv::launch_variant<2, 1, false, false, E>(tx, tw, ts, ty, d_bias, n_tiles, 1, 0, nullptr, n_boards, s, qo);
+    if (e != cudaSuccess) return fail(-2, "conv3x3_c256_kernel<e4m3> launch", e);
+    return 0;
+}
+
 int stem_lookup_impl(const char *name, const uint8_t *d_boards, int n, const int32_t *d_count, const void *d_table,
-                     const float *d_bias_turn, void *d_y, ccz_stream_t s) {
+                     const float *d_bias_turn, void *d_y, ccz_stream_t s, void *d_yq = nullptr, const float *d_inv_s = nullptr) {
     namespace st = ccz::stem;
     std::string e_name(name);
     if (n < 0) return fail(-1, (e_name + ": n < 0").c_str());
     if (n == 0) return 0;
     if (!d_boards || !d_table || !d_bias_turn || !d_y) return fail(-1, (e_name + ": NULL pointer").c_str());
-    if (((uintptr_t)d_boards & 3) || (((uintptr_t)d_table | (uintptr_t)d_bias_turn | (uintptr_t)d_y) & 15))
+    if (((uintptr_t)d_boards & 3) || (((uintptr_t)d_table | (uintptr_t)d_bias_turn | (uintptr_t)d_y | (uintptr_t)d_yq) & 15))
         return fail(-1, (e_name + ": pointers must be 16-byte aligned (boards 4-byte)").c_str());
     static int n_sm_dev[64] = {0};
     int dev = 0;
@@ -528,6 +577,8 @@ int stem_lookup_impl(const char *name, const uint8_t *d_boards, int n, const int
         CCZ_CUDA(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev));
         CCZ_CUDA(cudaFuncSetAttribute(st::stem_lookup_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, st::SMEM_BYTES));
         CCZ_CUDA(cudaFuncSetAttribute(st::stem_lookup_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, st::SMEM_BYTES));
+        CCZ_CUDA(cudaFuncSetAttribute(st::stem_lookup_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, st::SMEM_BYTES));
+        CCZ_CUDA(cudaFuncSetAttribute(st::stem_lookup_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, st::SMEM_BYTES));
     }
     int blocks = 2 * n_sm; // two resident CTAs (92 KB of tables each) per SM
     const int need = (n + st::WARPS - 1) / st::WARPS;
@@ -535,7 +586,13 @@ int stem_lookup_impl(const char *name, const uint8_t *d_boards, int n, const int
     const uint4 *tab = static_cast<const uint4 *>(d_table);
     const float4 *bt = reinterpret_cast<const float4 *>(d_bias_turn);
     uint4 *y = static_cast<uint4 *>(d_y);
-    if (d_count)
+    if (d_yq) {
+        uint2 *yq = static_cast<uint2 *>(d_yq);
+        if (d_count)
+            st::stem_lookup_kernel<true, true><<<blocks, st::WARPS * 32, st::SMEM_BYTES, s>>>(d_boards, n, tab, bt, y, d_count, yq, d_inv_s);
+        else
+            st::stem_lookup_kernel<false, true><<<blocks, st::WARPS * 32, st::SMEM_BYTES, s>>>(d_boards, n, tab, bt, y, nullptr, yq, d_inv_s);
+    } else if (d_count)
         st::stem_lookup_kernel<true><<<blocks, st::WARPS * 32, st::SMEM_BYTES, s>>>(d_boards, n, tab, bt, y, d_count);
     else
         st::stem_lookup_kernel<false><<<blocks, st::WARPS * 32, st::SMEM_BYTES, s>>>(d_boards, n, tab, bt, y, nullptr);
@@ -597,6 +654,18 @@ int ccz_stem_lookup_count(const uint8_t *d_boards, int capacity, const int32_t *
                           void *d_y, ccz_stream_t s) {
     if (!d_n_boards) return fail(-1, "ccz_stem_lookup_count: d_n_boards is NULL");
     return stem_lookup_impl("ccz_stem_lookup_count", d_boards, capacity, d_n_boards, d_table, d_bias_turn, d_y, s);
+}
+
+int ccz_conv3x3_c256_e4m3(const void *d_xq, const void *d_wq, const float *d_dequant, const float *d_bias, const void *d_skip, void *d_y,
+                          void *d_yq, const float *d_inv_s_out, int capacity, const int32_t *d_n_boards, ccz_stream_t s) {
+    return conv3x3_c256_e4m3_impl(d_xq, d_wq, d_dequant, d_bias, d_skip, d_y, d_yq, d_inv_s_out, capacity, d_n_boards, s);
+}
+
+int ccz_stem_lookup_e4m3(const uint8_t *d_boards, int capacity, const int32_t *d_n_boards, const void *d_table, const float *d_bias_turn,
+                         void *d_y, void *d_yq, const float *d_inv_s_out, ccz_stream_t s) {
+    if (!d_y || !d_yq || !d_inv_s_out) return fail(-1, "ccz_stem_lookup_e4m3: d_y, d_yq and d_inv_s_out are required");
+    if (d_yq == d_y) return fail(-1, "ccz_stem_lookup_e4m3: d_yq must not alias d_y");
+    return stem_lookup_impl("ccz_stem_lookup_e4m3", d_boards, capacity, d_n_boards, d_table, d_bias_turn, d_y, s, d_yq, d_inv_s_out);
 }
 
 int ccz_heads_pack(const void *d_h, int n, void *d_operands, int row_elems, int value_off, ccz_stream_t s) {

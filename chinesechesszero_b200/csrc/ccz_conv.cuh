@@ -16,6 +16,8 @@
 //   * Epilogue: 4 warps, one accumulator row per thread (tcgen05.ld 32x32b), + bias (+ skip, prefetched by
 //     TMA into the staging tile while the main loop runs) -> ReLU -> bf16 into the swizzled staging tile
 //     -> TMA store.
+//   * e4m3 variant (T = __nv_fp8_e4m3, the FP8 evaluator): kind::f8f6f4, 128 channels per 128-byte stage row,
+//     18 k-blocks, 4 stages; the epilogue dequantises per output channel and may write an e4m3 copy (QOut).
 // Warp roles (256 threads): 0 = A/B TMA producer, 1 = MMA issuer, 2 = TMEM allocator, 3 = skip-tile
 // producer, 4..7 = epilogue.
 //
@@ -36,9 +38,11 @@
 
 #include <cuda.h> // CUtensorMap + enums only; the encode functions are fetched at run time (no -lcuda)
 #include <cuda_bf16.h>
+#include <cuda_fp8.h>
 #include <cuda_runtime.h>
 
 #include <cstdint>
+#include <type_traits>
 
 #ifndef CCZ_CONV_BACKOFF_NS
 #define CCZ_CONV_BACKOFF_NS 256 // poll interval of the roles that wait a whole tile ahead
@@ -51,22 +55,45 @@ constexpr int C = 256;
 constexpr int BOARD_H = 10, BOARD_W = 9, BOARD_HW = 90;
 constexpr int BM = 128; // output pixels per CTA
 constexpr int BN = 256; // all output channels
-constexpr int BK = 64;  // one 128-byte swizzle row of bf16
-constexpr int KBLOCKS = 9 * (C / BK);
-constexpr int UMMA_K = 16;
 constexpr int THREADS = 256;
 
-template <int CG>
+// T = operand element type: __nv_bfloat16 (kind::f16) or __nv_fp8_e4m3 (kind::f8f6f4).  A stage is one 128-byte
+// swizzle row per operand row in both cases, so an e4m3 stage covers twice the K of a bf16 stage.
+template <int CG, typename T = __nv_bfloat16>
 struct Cfg {
+    static constexpr bool FP8 = std::is_same<T, __nv_fp8_e4m3>::value;
+    static constexpr int BK = 128 / (int)sizeof(T);     // channels per k-block
+    static constexpr int UMMA_K = 32 / (int)sizeof(T);  // K of one tcgen05.mma
+    static constexpr int CBLK_LOG2 = FP8 ? 1 : 2;       // log2(C / BK)
+    static constexpr int KBLOCKS = 9 << CBLK_LOG2;
     static constexpr int B_ROWS = BN / CG;
-    static constexpr int A_BYTES = BM * BK * 2;
-    static constexpr int B_BYTES = B_ROWS * BK * 2;
+    static constexpr int A_BYTES = BM * 128;
+    static constexpr int B_BYTES = B_ROWS * 128;
     static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
-    static constexpr int STAGES = CG == 2 ? 5 : 3;
-    static constexpr int STAGING_BYTES = BM * BN * 2; // 4 boxes of 128 rows x 64 channels
+    // e4m3: the dequant vector does not fit beside 5 stages (232,448 bytes a block); 4 e4m3 stages still cover more K
+    static constexpr int STAGES = CG == 2 ? (FP8 ? 4 : 5) : 3;
+    static constexpr int STAGING_BYTES = BM * BN * 2; // 4 boxes of 128 rows x 64 bf16 channels
     static constexpr int BIAS_BYTES = BN * 4;
+    static constexpr int DEQ_BYTES = FP8 ? BN * 4 : 0;
     static constexpr int BAR_BYTES = 256;
-    static constexpr int SMEM_BYTES = 1024 /*alignment slack*/ + STAGES * STAGE_BYTES + STAGING_BYTES + BIAS_BYTES + BAR_BYTES;
+    static constexpr int SMEM_BYTES =
+        1024 /*alignment slack*/ + STAGES * STAGE_BYTES + STAGING_BYTES + BIAS_BYTES + DEQ_BYTES + BAR_BYTES;
+};
+static_assert(Cfg<2, __nv_fp8_e4m3>::SMEM_BYTES <= 232448 && Cfg<2>::SMEM_BYTES <= 232448, "shared memory budget");
+
+// Extra epilogue operands of the e4m3 kernel (empty for bf16):
+//   f = acc * dequant[co] + bias[co] (+ skip) -> ReLU;  y = bf16(f) when out_y;  yq = e4m3 satfinite(f * *inv_s_out)
+// yq is written straight from registers (a thread owns one pixel's 256 contiguous bytes); inv_s_out is read on the
+// device so that a captured graph follows refreshed scales.
+template <typename T>
+struct QOut {};
+template <>
+struct QOut<__nv_fp8_e4m3> {
+    const float *dequant;   // [256] s_in * s_w[co]
+    uint8_t *yq;            // e4m3 [rows, 256] or nullptr
+    const float *inv_s_out; // scalar, read when yq != nullptr
+    long long rows;         // output rows the tensor maps cover (capacity * 90)
+    int out_y;              // write the bf16 y
 };
 
 // ---- PTX wrappers ---------------------------------------------------------------------------
@@ -226,6 +253,23 @@ __device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a_desc, uint
             : "memory");
     }
 }
+// D[tmem] (+)= A[smem] * B[smem]^T, e4m3 x e4m3 -> fp32
+template <int CG>
+__device__ __forceinline__ void umma_e4m3(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
+    if constexpr (CG == 1) {
+        asm volatile(
+            "{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\n"
+            "tcgen05.mma.cta_group::1.kind::f8f6f4 [%0], %1, %2, %3, p;\n}" ::"r"(d_tmem),
+            "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+            : "memory");
+    } else {
+        asm volatile(
+            "{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\n"
+            "tcgen05.mma.cta_group::2.kind::f8f6f4 [%0], %1, %2, %3, p;\n}" ::"r"(d_tmem),
+            "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+            : "memory");
+    }
+}
 // arrive on `bar` (same offset in every CTA of the pair) once all MMAs issued so far have completed
 template <int CG>
 __device__ __forceinline__ void umma_commit(uint32_t bar, uint16_t cta_mask) {
@@ -270,14 +314,22 @@ __device__ __forceinline__ void cluster_sync_all() {
 __device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr) {
     return (uint64_t)((smem_addr >> 4) & 0x3FFF) | (1ull << 16) | (64ull << 32) | (1ull << 46) | (2ull << 61);
 }
-// instruction descriptor: fp32 accumulate [4,6)=1, A/B bf16 [7,10)=[10,13)=1, both K-major, N>>3 at 17, M>>4 at 24
-__host__ __device__ constexpr uint32_t umma_idesc(int m, int n) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
+// instruction descriptor: fp32 accumulate [4,6)=1, A/B format [7,10)=[10,13) (kind::f16: 1 = bf16; kind::f8f6f4: 0 = e4m3),
+// both K-major, N>>3 at 17, M>>4 at 24
+__host__ __device__ constexpr uint32_t umma_idesc(int m, int n, uint32_t ab_fmt = 1) {
+    return (1u << 4) | (ab_fmt << 7) | (ab_fmt << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
 }
 
 __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
     __nv_bfloat162 t = __floats2bfloat162_rn(lo, hi);
     return *reinterpret_cast<uint32_t *>(&t);
+}
+// four floats -> four e4m3 (round to nearest even, saturated to +-448; a NaN stays NaN), a in the lowest byte
+__device__ __forceinline__ uint32_t pack_e4m3x4(float a, float b, float c, float d) {
+    uint16_t lo, hi;
+    asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(lo) : "f"(b), "f"(a));
+    asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(hi) : "f"(d), "f"(c));
+    return (uint32_t)lo | ((uint32_t)hi << 16);
 }
 
 // ---- the kernel --------------------------------------------------------------------------------
@@ -320,19 +372,23 @@ __host__ __device__ inline Plan plan_items(int n_tiles, int clusters, bool tail_
 // DEV_COUNT: the board count is read from device memory (min(*d_count, count_cap), the tensor maps being encoded for
 // count_cap boards), and every CTA derives the plan from it as the host does; the grid is every resident cluster and
 // the clusters without an item only allocate / free TMEM and pass the cluster barriers.
-template <int CG, int PAIRS, bool HAS_SKIP, bool DEV_COUNT>
+//
+// T = __nv_fp8_e4m3: x and w are e4m3, the accumulator is dequantised per output channel in the epilogue (QOut).
+template <int CG, int PAIRS, bool HAS_SKIP, bool DEV_COUNT, typename T = __nv_bfloat16>
 __global__ void __launch_bounds__(THREADS, 1)
 conv3x3_c256_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUtensorMap tm_w,
                     const __grid_constant__ CUtensorMap tm_skip, const __grid_constant__ CUtensorMap tm_y, const float *__restrict__ bias,
-                    int n_items, int n_full, int split_log2, int dbg, const int32_t *__restrict__ d_count, int count_cap, int tail_split) {
-    using K = Cfg<CG>;
+                    int n_items, int n_full, int split_log2, int dbg, const int32_t *__restrict__ d_count, int count_cap, int tail_split,
+                    const QOut<T> qo) {
+    using K = Cfg<CG, T>;
     extern __shared__ uint8_t smem_raw[];
     const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
     const uint32_t a_smem = smem_base;
     const uint32_t b_smem = a_smem + K::STAGES * K::A_BYTES;
     const uint32_t staging = b_smem + K::STAGES * K::B_BYTES;
     const uint32_t bias_smem = staging + K::STAGING_BYTES;
-    const uint32_t bars = bias_smem + K::BIAS_BYTES;
+    const uint32_t deq_smem = bias_smem + K::BIAS_BYTES; // e4m3 only
+    const uint32_t bars = deq_smem + K::DEQ_BYTES;
     const uint32_t bar_full = bars;                      // [STAGES]
     const uint32_t bar_empty = bars + 8 * K::STAGES;     // [STAGES]
     const uint32_t bar_tfull = bars + 16 * K::STAGES;    // [2]
@@ -380,6 +436,10 @@ conv3x3_c256_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
         const int t = threadIdx.x - 128;
         reinterpret_cast<float *>(smem_gen + (bias_smem - smem_base))[t] = bias[t];
         reinterpret_cast<float *>(smem_gen + (bias_smem - smem_base))[t + 128] = bias[t + 128];
+        if constexpr (K::FP8) {
+            reinterpret_cast<float *>(smem_gen + (deq_smem - smem_base))[t] = qo.dequant[t];
+            reinterpret_cast<float *>(smem_gen + (deq_smem - smem_base))[t + 128] = qo.dequant[t + 128];
+        }
     }
     tc_fence_before();
     if constexpr (CLUSTER > 1) cluster_sync_all(); else __syncthreads();
@@ -401,17 +461,17 @@ conv3x3_c256_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
                 const int b_row = wi.n_off + (int)prank * (wi.n_w / CG); // a channel slice over-reads rows it does not use
                 const int img = m0 / BOARD_HW, rem = m0 - img * BOARD_HW;
                 const int p = rem / BOARD_W, q = rem - p * BOARD_W;
-                for (int kb = 0; kb < KBLOCKS; ++kb) {
-                    const int tap = kb >> 2, c0 = (kb & 3) * BK;
+                for (int kb = 0; kb < K::KBLOCKS; ++kb) {
+                    const int tap = kb >> K::CBLK_LOG2, c0 = (kb & ((1 << K::CBLK_LOG2) - 1)) * K::BK;
                     const int r = tap / 3, s = tap - 3 * r;
                     mbar_wait(bar_empty + 8 * stage, phase ^ 1);
                     const bool do_a = !((dbg & 2) && (kb & 1)), do_b = !((dbg & 1) && (kb & 1)); // traffic-sensitivity experiment
                     if (prank == 0) mbar_expect_tx(bar_full + 8 * stage, CG * ((do_a ? K::A_BYTES : 0) + (do_b ? K::B_BYTES : 0)));
                     if (do_a) tma_load_im2col<CG>(a_smem + stage * K::A_BYTES, &tm_x, full0 + 8 * stage, c0, q - 1, p - 1, img, (uint16_t)s, (uint16_t)r);
                     if constexpr (PAIRS == 1) {
-                        if (do_b) tma_load_2d<CG>(b_smem + stage * K::B_BYTES, &tm_w, full0 + 8 * stage, kb * BK, b_row);
+                        if (do_b) tma_load_2d<CG>(b_smem + stage * K::B_BYTES, &tm_w, full0 + 8 * stage, kb * K::BK, b_row);
                     } else {
-                        tma_load_2d_mc(b_smem + stage * K::B_BYTES + (int)pair_id * SLICE_ROWS * 128, &tm_w, full0 + 8 * stage, kb * BK,
+                        tma_load_2d_mc(b_smem + stage * K::B_BYTES + (int)pair_id * SLICE_ROWS * 128, &tm_w, full0 + 8 * stage, kb * K::BK,
                                        b_row + (int)pair_id * SLICE_ROWS, mc_mask);
                     }
                     if (++stage == K::STAGES) { stage = 0; phase ^= 1; }
@@ -426,18 +486,22 @@ conv3x3_c256_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
             int stage = 0;
             uint32_t phase = 0, acc = 0, acc_phase = 0;
             for (int item = cluster_id; item < n_items; item += n_clusters) {
-                const uint32_t idesc = umma_idesc(BM * CG, work_item(item, n_full, split_log2).n_w);
+                const uint32_t idesc = umma_idesc(BM * CG, work_item(item, n_full, split_log2).n_w, K::FP8 ? 0u : 1u);
                 mbar_wait_cluster(bar_tempty + 8 * acc, acc_phase ^ 1);
                 tc_fence_after();
                 const uint32_t d_tmem = tmem_base + acc * BN;
-                for (int kb = 0; kb < KBLOCKS; ++kb) {
+                for (int kb = 0; kb < K::KBLOCKS; ++kb) {
                     mbar_wait(bar_full + 8 * stage, phase);
                     tc_fence_after();
                     const uint64_t a_desc = umma_desc_sw128(a_smem + stage * K::A_BYTES);
                     const uint64_t b_desc = umma_desc_sw128(b_smem + stage * K::B_BYTES);
 #pragma unroll
-                    for (int k = 0; k < BK / UMMA_K; ++k) // +32 bytes along K inside the swizzle row
-                        umma_bf16<CG>(d_tmem, a_desc + 2 * k, b_desc + 2 * k, idesc, (uint32_t)((kb | k) != 0));
+                    for (int k = 0; k < K::BK / K::UMMA_K; ++k) { // +32 bytes along K inside the swizzle row
+                        if constexpr (K::FP8)
+                            umma_e4m3<CG>(d_tmem, a_desc + 2 * k, b_desc + 2 * k, idesc, (uint32_t)((kb | k) != 0));
+                        else
+                            umma_bf16<CG>(d_tmem, a_desc + 2 * k, b_desc + 2 * k, idesc, (uint32_t)((kb | k) != 0));
+                    }
                     umma_commit<CG>(bar_empty + 8 * stage, mask_cluster);
                     if (++stage == K::STAGES) { stage = 0; phase ^= 1; }
                 }
@@ -463,6 +527,11 @@ conv3x3_c256_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
         const uint32_t tempty0 = CG == 2 ? mapa(bar_tempty, lead_rank) : bar_tempty;
         const float *bias_s = reinterpret_cast<const float *>(smem_gen + (bias_smem - smem_base));
         uint8_t *stg = smem_gen + (staging - smem_base);
+        [[maybe_unused]] const float *deq_s = reinterpret_cast<const float *>(smem_gen + (deq_smem - smem_base));
+        [[maybe_unused]] float inv_s = 0.f;
+        if constexpr (K::FP8) {
+            if (qo.yq) inv_s = *qo.inv_s_out;
+        }
         uint32_t acc = 0, acc_phase = 0, it = 0;
         for (int item = cluster_id; item < n_items; item += n_clusters, ++it) {
             const WorkItem wi = work_item(item, n_full, split_log2);
@@ -477,16 +546,27 @@ conv3x3_c256_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
                 tmem_ld32(t_row + chunk * 32, v);
                 tmem_ld_wait();
                 uint8_t *box_row = stg + (chunk >> 1) * (BM * 128) + row * 128;
+                [[maybe_unused]] uint32_t q[8]; // e4m3: the chunk's 32 output bytes
 #pragma unroll
                 for (int j = 0; j < 4; ++j) {
                     const int c16 = (chunk & 1) * 4 + j; // 16-byte column of the 128-byte row
                     uint4 *cell = reinterpret_cast<uint4 *>(box_row + ((c16 ^ (row & 7)) << 4));
                     const float4 b0 = *reinterpret_cast<const float4 *>(bias_s + wi.n_off + chunk * 32 + j * 8);
                     const float4 b1 = *reinterpret_cast<const float4 *>(bias_s + wi.n_off + chunk * 32 + j * 8 + 4);
-                    float f[8] = {__uint_as_float(v[j * 8 + 0]) + b0.x, __uint_as_float(v[j * 8 + 1]) + b0.y,
-                                  __uint_as_float(v[j * 8 + 2]) + b0.z, __uint_as_float(v[j * 8 + 3]) + b0.w,
-                                  __uint_as_float(v[j * 8 + 4]) + b1.x, __uint_as_float(v[j * 8 + 5]) + b1.y,
-                                  __uint_as_float(v[j * 8 + 6]) + b1.z, __uint_as_float(v[j * 8 + 7]) + b1.w};
+                    float f[8];
+                    if constexpr (K::FP8) {
+                        const float4 d0 = *reinterpret_cast<const float4 *>(deq_s + wi.n_off + chunk * 32 + j * 8);
+                        const float4 d1 = *reinterpret_cast<const float4 *>(deq_s + wi.n_off + chunk * 32 + j * 8 + 4);
+                        const float d[8] = {d0.x, d0.y, d0.z, d0.w, d1.x, d1.y, d1.z, d1.w};
+                        const float b[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
+#pragma unroll
+                        for (int e = 0; e < 8; ++e) f[e] = fmaf(__uint_as_float(v[j * 8 + e]), d[e], b[e]);
+                    } else {
+                        f[0] = __uint_as_float(v[j * 8 + 0]) + b0.x; f[1] = __uint_as_float(v[j * 8 + 1]) + b0.y;
+                        f[2] = __uint_as_float(v[j * 8 + 2]) + b0.z; f[3] = __uint_as_float(v[j * 8 + 3]) + b0.w;
+                        f[4] = __uint_as_float(v[j * 8 + 4]) + b1.x; f[5] = __uint_as_float(v[j * 8 + 5]) + b1.y;
+                        f[6] = __uint_as_float(v[j * 8 + 6]) + b1.z; f[7] = __uint_as_float(v[j * 8 + 7]) + b1.w;
+                    }
                     if (HAS_SKIP) {
                         const uint4 sk = *cell;
                         const uint32_t w[4] = {sk.x, sk.y, sk.z, sk.w};
@@ -496,12 +576,28 @@ conv3x3_c256_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
                             f[2 * e + 1] += __uint_as_float(w[e] & 0xFFFF0000u);
                         }
                     }
-                    uint4 o;
-                    o.x = pack_bf16x2(fmaxf(f[0], 0.f), fmaxf(f[1], 0.f));
-                    o.y = pack_bf16x2(fmaxf(f[2], 0.f), fmaxf(f[3], 0.f));
-                    o.z = pack_bf16x2(fmaxf(f[4], 0.f), fmaxf(f[5], 0.f));
-                    o.w = pack_bf16x2(fmaxf(f[6], 0.f), fmaxf(f[7], 0.f));
-                    *cell = o;
+                    if constexpr (K::FP8) {
+#pragma unroll
+                        for (int e = 0; e < 8; ++e) f[e] = fmaxf(f[e], 0.f);
+                        if (qo.out_y) *cell = make_uint4(pack_bf16x2(f[0], f[1]), pack_bf16x2(f[2], f[3]), pack_bf16x2(f[4], f[5]),
+                                                         pack_bf16x2(f[6], f[7]));
+                        q[2 * j] = pack_e4m3x4(f[0] * inv_s, f[1] * inv_s, f[2] * inv_s, f[3] * inv_s);
+                        q[2 * j + 1] = pack_e4m3x4(f[4] * inv_s, f[5] * inv_s, f[6] * inv_s, f[7] * inv_s);
+                    } else {
+                        uint4 o;
+                        o.x = pack_bf16x2(fmaxf(f[0], 0.f), fmaxf(f[1], 0.f));
+                        o.y = pack_bf16x2(fmaxf(f[2], 0.f), fmaxf(f[3], 0.f));
+                        o.z = pack_bf16x2(fmaxf(f[4], 0.f), fmaxf(f[5], 0.f));
+                        o.w = pack_bf16x2(fmaxf(f[6], 0.f), fmaxf(f[7], 0.f));
+                        *cell = o;
+                    }
+                }
+                if constexpr (K::FP8) {
+                    if (qo.yq && m0 + row < qo.rows) {
+                        uint4 *dst = reinterpret_cast<uint4 *>(qo.yq + (size_t)(m0 + row) * C + wi.n_off + chunk * 32);
+                        dst[0] = make_uint4(q[0], q[1], q[2], q[3]);
+                        dst[1] = make_uint4(q[4], q[5], q[6], q[7]);
+                    }
                 }
             }
             // accumulator buffer drained: hand it back to the MMA issuer
@@ -515,7 +611,10 @@ conv3x3_c256_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
             fence_proxy_async();
             asm volatile("bar.sync 1, 128;" ::: "memory");
             if (threadIdx.x == 128) {
-                for (int g = 0; g < wi.n_w / 64; ++g) tma_store_2d(&tm_y, staging + g * (BM * 128), wi.n_off + g * 64, m0);
+                bool store_y = true;
+                if constexpr (K::FP8) store_y = qo.out_y != 0;
+                if (store_y)
+                    for (int g = 0; g < wi.n_w / 64; ++g) tma_store_2d(&tm_y, staging + g * (BM * 128), wi.n_off + g * 64, m0);
                 tma_store_commit();
                 tma_store_wait_read();
                 if (HAS_SKIP) mbar_arrive(bar_stfree);
@@ -564,34 +663,41 @@ inline const char *driver_init(Driver &d) {
     return nullptr;
 }
 
-// [rows, 256] bf16 row-major matrix, box = 64 channels x box_rows rows, 128-byte swizzle
-inline bool encode_rows(const Driver &d, CUtensorMap *m, const void *ptr, uint64_t rows, uint64_t cols, uint32_t box_rows) {
+// [rows, cols] row-major matrix of bf16 (or e4m3 as UINT8), box = one 128-byte row x box_rows rows, 128-byte swizzle
+inline bool encode_rows(const Driver &d, CUtensorMap *m, const void *ptr, uint64_t rows, uint64_t cols, uint32_t box_rows,
+                        bool e4m3 = false) {
+    const uint64_t esz = e4m3 ? 1 : 2;
     const cuuint64_t dims[2] = {cols, rows};
-    const cuuint64_t strides[1] = {cols * 2};
-    const cuuint32_t box[2] = {64, box_rows};
+    const cuuint64_t strides[1] = {cols * esz};
+    const cuuint32_t box[2] = {(cuuint32_t)(128 / esz), box_rows};
     const cuuint32_t es[2] = {1, 1};
-    return d.tiled(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void *>(ptr), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
+    return d.tiled(m, e4m3 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void *>(ptr), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
                    CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
 // NHWC activations [n,10,9,256] for a 3x3 / pad 1 fprop: base pixels span [-1, dim-1+(-1)] in w and h,
-// the filter tap is added by the instruction's offsets; 64 channels x 128 pixels per load.
-inline bool encode_im2col(const Driver &d, CUtensorMap *m, const void *ptr, int n) {
+// the filter tap is added by the instruction's offsets; one 128-byte row of channels (64 bf16 / 128 e4m3) x 128 pixels
+// per load.
+inline bool encode_im2col(const Driver &d, CUtensorMap *m, const void *ptr, int n, bool e4m3 = false) {
+    const cuuint64_t esz = e4m3 ? 1 : 2;
     const cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)BOARD_W, (cuuint64_t)BOARD_H, (cuuint64_t)n};
-    const cuuint64_t strides[3] = {(cuuint64_t)C * 2, (cuuint64_t)C * 2 * BOARD_W, (cuuint64_t)C * 2 * BOARD_HW};
+    const cuuint64_t strides[3] = {(cuuint64_t)C * esz, (cuuint64_t)C * esz * BOARD_W, (cuuint64_t)C * esz * BOARD_HW};
     const int lower[2] = {-1, -1}, upper[2] = {-1, -1};
     const cuuint32_t es[4] = {1, 1, 1, 1};
-    return d.im2col(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void *>(ptr), dims, strides, lower, upper, BK, BM, es,
+    return d.im2col(m, e4m3 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void *>(ptr), dims, strides,
+                    lower, upper, (cuuint32_t)(128 / esz), BM, es,
                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
 // d_count == nullptr: `n_tiles` cluster tiles planned here.  Otherwise the kernel plans from min(*d_count, count_cap)
 // boards on the device and every resident cluster is launched.
-template <int CG, int PAIRS, bool HAS_SKIP, bool DEV_COUNT>
+template <int CG, int PAIRS, bool HAS_SKIP, bool DEV_COUNT, typename T = __nv_bfloat16>
 inline cudaError_t launch_variant(const CUtensorMap &tx, const CUtensorMap &tw, const CUtensorMap &ts, const CUtensorMap &ty, const float *bias,
-                                  int n_tiles, int tail_split, int dbg, const int32_t *d_count, int count_cap, cudaStream_t stream) {
-    auto kern = conv3x3_c256_kernel<CG, PAIRS, HAS_SKIP, DEV_COUNT>;
+                                  int n_tiles, int tail_split, int dbg, const int32_t *d_count, int count_cap, cudaStream_t stream,
+                                  const QOut<T> &qo = {}) {
+    using K = Cfg<CG, T>;
+    auto kern = conv3x3_c256_kernel<CG, PAIRS, HAS_SKIP, DEV_COUNT, T>;
     constexpr int CLUSTER = CG * PAIRS;
     // per device: resident clusters of this shape (GPC boundaries can strand SMs for CLUSTER > 2); function
     // attributes are per device too
@@ -603,7 +709,7 @@ inline cudaError_t launch_variant(const CUtensorMap &tx, const CUtensorMap &tw, 
     int &max_clusters = max_clusters_dev[dev];
     cudaLaunchConfig_t cfg = {};
     cfg.blockDim = dim3(THREADS);
-    cfg.dynamicSmemBytes = Cfg<CG>::SMEM_BYTES;
+    cfg.dynamicSmemBytes = K::SMEM_BYTES;
     cfg.stream = stream;
     cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeClusterDimension;
@@ -615,7 +721,7 @@ inline cudaError_t launch_variant(const CUtensorMap &tx, const CUtensorMap &tw, 
     if (!max_clusters) {
         cudaError_t e = cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
         if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<CG>::SMEM_BYTES);
+        e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, K::SMEM_BYTES);
         if (e != cudaSuccess) return e;
         cfg.gridDim = dim3((unsigned)(n_sm / CLUSTER * CLUSTER));
         int n = 0;
@@ -626,11 +732,12 @@ inline cudaError_t launch_variant(const CUtensorMap &tx, const CUtensorMap &tw, 
     }
     if constexpr (DEV_COUNT) {
         cfg.gridDim = dim3((unsigned)(max_clusters * CLUSTER));
-        return cudaLaunchKernelEx(&cfg, kern, tx, tw, ts, ty, bias, 0, 0, 0, dbg, d_count, count_cap, tail_split);
+        return cudaLaunchKernelEx(&cfg, kern, tx, tw, ts, ty, bias, 0, 0, 0, dbg, d_count, count_cap, tail_split, qo);
     }
     const Plan pl = plan_items(n_tiles, max_clusters, tail_split != 0);
     cfg.gridDim = dim3((unsigned)(pl.clusters * CLUSTER));
-    return cudaLaunchKernelEx(&cfg, kern, tx, tw, ts, ty, bias, pl.n_items, pl.n_full, pl.split_log2, dbg, (const int32_t *)nullptr, 0, 0);
+    return cudaLaunchKernelEx(&cfg, kern, tx, tw, ts, ty, bias, pl.n_items, pl.n_full, pl.split_log2, dbg, (const int32_t *)nullptr, 0, 0,
+                              qo);
 }
 
 } // namespace conv

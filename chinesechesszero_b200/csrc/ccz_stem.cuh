@@ -14,13 +14,16 @@
 // No planes are read (21 KB / position saved), no channel padding, no layout copy: the kernel is bound by
 // the 46 KB / board NHWC bf16 output it writes.  One warp per board, lane = 8 output channels; tables
 // (92 KB) staged in shared memory once per persistent CTA.  DEV_COUNT: the board count is min(*d_count, n), read
-// on the device (K12's number of distinct leaves); warps past it exit.
+// on the device (K12's number of distinct leaves); warps past it exit.  QOUT: also an e4m3 copy of the output,
+// yq = satfinite(bf16(y) * *inv_s) (the A operand of the first e4m3 tower convolution; the bf16 y stays the skip).
 #pragma once
 
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 
 #include <cstdint>
+
+#include "ccz_conv.cuh" // pack_e4m3x4
 
 namespace ccz {
 namespace stem {
@@ -41,11 +44,14 @@ __device__ __forceinline__ void add_row(float (&acc)[8], const uint4 t) {
     }
 }
 
-template <bool DEV_COUNT>
+template <bool DEV_COUNT, bool QOUT = false>
 __global__ void __launch_bounds__(WARPS * 32, 2)
 stem_lookup_kernel(const uint8_t *__restrict__ boards, int n, const uint4 *__restrict__ table, const float4 *__restrict__ bias_turn,
-                   uint4 *__restrict__ y, const int32_t *__restrict__ d_count) {
+                   uint4 *__restrict__ y, const int32_t *__restrict__ d_count, uint2 *__restrict__ yq = nullptr,
+                   const float *__restrict__ inv_s = nullptr) {
     if constexpr (DEV_COUNT) n = min(*d_count, n);
+    [[maybe_unused]] float qs = 0.f;
+    if constexpr (QOUT) qs = *inv_s;
     extern __shared__ __align__(16) uint8_t smem[];
     uint4 *tab_s = reinterpret_cast<uint4 *>(smem);
     float4 *bt_s = reinterpret_cast<float4 *>(smem + TABLE_ELEMS * 2);
@@ -109,6 +115,13 @@ stem_lookup_kernel(const uint8_t *__restrict__ boards, int n, const uint4 *__res
                 o.z = *reinterpret_cast<uint32_t *>(&p2);
                 o.w = *reinterpret_cast<uint32_t *>(&p3);
                 out[(h * 9 + w) * (C_OUT / 8)] = o; // 32 lanes x 16 B = one 512-byte NHWC pixel row
+                if constexpr (QOUT) {
+                    const float2 f0 = __bfloat1622float2(p0), f1 = __bfloat1622float2(p1), f2 = __bfloat1622float2(p2),
+                                 f3 = __bfloat1622float2(p3);
+                    yq[((size_t)b * 90 + h * 9 + w) * (C_OUT / 8) + lane] =
+                        make_uint2(conv::pack_e4m3x4(f0.x * qs, f0.y * qs, f1.x * qs, f1.y * qs),
+                                   conv::pack_e4m3x4(f2.x * qs, f2.y * qs, f3.x * qs, f3.y * qs));
+                }
             }
         }
     }

@@ -25,6 +25,55 @@ PLAYS = 17  # net.py:13
 N_ACTIONS = _lib.N_ACTIONS
 # conv + linear multiply-accumulates of one forward, x2 (SURVEY.md §6): 8.5506 GFLOP / position
 FLOP_PER_POSITION = 2 * 4_275_314_716
+PRECISIONS = ("bf16", "fp8")
+E4M3_MAX = 448.0  # largest finite float8_e4m3fn
+
+
+def e4m3_quantize(x: torch.Tensor, inv_scale) -> torch.Tensor:
+    """``satfinite(x * inv_scale)`` in float8_e4m3fn: fp32 product, clamped to +-448, rounded to nearest even -- what the
+    kernels' ``cvt.rn.satfinite.e4m3x2.f32`` computes (torch's cast alone turns values past 448 into NaN)."""
+    q = (x.float() * inv_scale).clamp_(-E4M3_MAX, E4M3_MAX).to(torch.float8_e4m3fn)
+    return q.contiguous(memory_format=torch.channels_last) if q.dim() == 4 else q
+
+
+def weight_scales(w: torch.Tensor) -> torch.Tensor:
+    """Per-output-channel e4m3 scales of a folded weight ``w`` (co, ...): ``amax|w[co]| / 448`` (1 for an all-zero channel)."""
+    amax = w.detach().float().abs().flatten(1).amax(1)
+    return torch.where(amax > 0, amax / E4M3_MAX, torch.ones_like(amax))
+
+
+def activation_scale(amax: torch.Tensor) -> torch.Tensor:
+    """Static per-tensor e4m3 scale from a calibration amax: ``amax / 448`` (1 where amax is 0)."""
+    amax = amax.float()
+    return torch.where(amax > 0, amax / E4M3_MAX, torch.ones_like(amax))
+
+
+def calibration_boards(n: int = 1024, seed: int = 0, device="cuda") -> torch.Tensor:
+    """Fixed seeded calibration positions for the FP8 evaluator, generated on the device with K1 / K2: half a seeded sample
+    of the perft-4 leaves (the openings self-play starts from), half the ends of seeded uniform random playouts of 8..80
+    plies (middle games and endgames)."""
+    from . import positions
+
+    rng = np.random.default_rng(seed)
+    l4 = positions.perft_levels(4, device)[3]
+    n_open = n // 2
+    pick = np.sort(rng.choice(l4.shape[0], size=n_open, replace=False))
+    opening = l4[torch.from_numpy(pick).to(l4.device)].contiguous()
+    del l4
+    boards = _lib.boards_start(n - n_open, device)
+    depth = torch.from_numpy(rng.integers(8, 81, size=n - n_open)).to(boards.device)
+    for ply in range(80):
+        ids, counts, _, _ = _lib.movegen_encode(boards, planes=False)
+        u = torch.from_numpy(rng.random(boards.shape[0], dtype=np.float32)).to(boards.device)
+        active = ((counts > 0) & (depth > ply)).nonzero().view(-1)
+        if active.numel() == 0:
+            break
+        c = counts[active].to(torch.int64)
+        slot = torch.minimum((u[active] * c).to(torch.int64), c - 1)
+        sub = boards[active].contiguous()
+        _lib.board_push(sub, ids[active, slot].contiguous(), None)
+        boards[active] = sub
+    return torch.cat([opening, boards]).contiguous()
 
 
 class ResBlock(nn.Module):
@@ -124,6 +173,13 @@ class BatchedEvaluator:
     compacts the leaf batch to its U distinct positions; K10 and K9 then run on U boards (the count stays on the
     device), the 1x1 heads GEMM on the compacted buffer, and K11 packs each game's FC operands from its position's
     row.  Results are bit-identical to ``dedup=False``: every board's forward output is independent of its row.
+
+    ``precision="fp8"`` (opt-in; needs ``conv_impl="k9"`` and the 256-channel tower) runs the 80 tower convolutions on the
+    e4m3 variant of K9: operands in float8_e4m3fn, fp32 accumulation, bf16 residual stream, heads and FC layers unchanged.
+    Weights get one scale per output channel; activations one static scale per tensor from a calibration forward of the
+    bf16 tower over ``calib_boards`` ((n,96) board records; default :func:`calibration_boards`).  ``refresh`` re-quantises
+    and re-calibrates in place, so captured graphs replay with the new weights and scales.  Check the strength of a
+    trained net in fp8 against bf16 with ``evaluate.EvaluationMatch(ev_fp8, ev_bf16, ...)``.
     """
 
     #: which kernel runs the 3x3 tower convolutions:
@@ -135,9 +191,13 @@ class BatchedEvaluator:
     CONV_IMPLS = ("k9", "k9_skip", "cudnn", "torch")
 
     def __init__(self, net: Net, device="cuda", dtype=torch.bfloat16, fused_epilogue: bool = True,
-                 conv_impl: str | None = None, chunk: int | None = None, dedup: bool = True):
+                 conv_impl: str | None = None, chunk: int | None = None, dedup: bool = True, precision: str = "bf16",
+                 calib_boards: torch.Tensor | None = None):
         self.device = torch.device(device)
         self.dtype = dtype
+        if precision not in PRECISIONS:
+            raise ValueError(f"precision must be one of {PRECISIONS}")
+        self.precision = precision
         # leaves per sub-batch (0 = whole batch at once): sub-batches whose activations fit the 126 MB L2
         # keep the tower's layer-to-layer traffic out of HBM
         self.chunk = int(os.environ.get("CCZ_EVAL_CHUNK", "0")) if chunk is None else int(chunk)
@@ -146,6 +206,8 @@ class BatchedEvaluator:
         if conv_impl not in self.CONV_IMPLS:
             raise ValueError(f"conv_impl must be one of {self.CONV_IMPLS}")
         k9_ok = self.device.type == "cuda" and dtype == torch.bfloat16 and net.conv_block.out_channels == 256
+        if precision == "fp8" and not (conv_impl == "k9" and k9_ok):
+            raise ValueError('precision="fp8" needs conv_impl="k9", a CUDA device, dtype bfloat16 and a 256-channel net')
         if conv_impl in ("k9", "k9_skip") and not k9_ok:
             conv_impl = "cudnn"  # K9 is specialised for the 256-channel bf16 tower of the reference net
         self.conv_impl = conv_impl
@@ -160,6 +222,13 @@ class BatchedEvaluator:
         # measurement hook (bench.py): when a list, every K9 launch of the next forwards is bracketed by CUDA
         # events on the launching stream and the (with_skip, start, end) triples are appended to it
         self.conv_events: list | None = None
+        if precision == "fp8":
+            if calib_boards is None:
+                calib_boards = calibration_boards(device=self.device)
+            elif calib_boards.dtype != torch.uint8 or calib_boards.dim() != 2 or calib_boards.shape[1] != _lib.BOARD_BYTES \
+                    or calib_boards.shape[0] < 1:
+                raise ValueError("calib_boards must be uint8 (n,96) board records, n >= 1")
+            self.calib_boards = calib_boards.to(self.device).contiguous()
         self.refresh(net)
 
     def _keep(self, key: str, t: torch.Tensor) -> torch.Tensor:
@@ -227,6 +296,50 @@ class BatchedEvaluator:
         self._heads_gemm = (keep("heads.gemm_w", hw), keep("heads.gemm_b", hb))
         self.value_fc2 = (keep("vfc2.w", net.value_fc2.weight.detach().to(dev, torch.float32).clone()),
                           keep("vfc2.b", net.value_fc2.bias.detach().to(dev, torch.float32).clone()))
+        if self.precision == "fp8":
+            self._refresh_fp8(net)
+
+    def _refresh_fp8(self, net: Net) -> None:
+        """e4m3 tower operands: per-channel weight scales on the fp32 folded weights, static activation scales from a
+        calibration forward of the bf16 tower (K10 + K9) over ``calib_boards``."""
+        keep, dev, cl = self._keep, self.device, torch.channels_last
+        amax_x, amax_y = [], []  # block inputs x_l and conv1 outputs y_l (post-ReLU, so amax = max)
+        for i in range(0, self.calib_boards.shape[0], 4096):
+            x = _lib.stem_lookup(self.calib_boards[i:i + 4096], *self.stem_lookup)
+            ax, ay = [], []
+            for (w1, _, b1), (w2, _, b2) in self.blocks:
+                ax.append(x.amax())
+                y = _lib.conv3x3_c256(x, w1, b1)
+                ay.append(y.amax())
+                x = _lib.conv3x3_c256(y, w2, b2, skip=x, out=x)
+            amax_x.append(torch.stack(ax).float())
+            amax_y.append(torch.stack(ay).float())
+        s_x = activation_scale(torch.stack(amax_x).amax(0))
+        s_y = activation_scale(torch.stack(amax_y).amax(0))
+        self.fp8_scales = {"x": keep("fp8.s_x", s_x), "y": keep("fp8.s_y", s_y)}
+        self._inv_sx, self._inv_sy = keep("fp8.inv_sx", 1.0 / s_x), keep("fp8.inv_sy", 1.0 / s_y)
+        self.qblocks = []
+        for i, rb in enumerate(net.res_blocks):
+            convs = []
+            for j, (conv, bn, s_in) in enumerate(((rb.conv1, rb.conv1_bn, s_x[i]), (rb.conv2, rb.conv2_bn, s_y[i])), 1):
+                w, _ = _fold(conv, bn)
+                w = w.to(dev)
+                s_w = weight_scales(w)
+                wq = e4m3_quantize(w, (1.0 / s_w).view(-1, 1, 1, 1))
+                convs.append((keep(f"rb{i}.{j}.wq", wq.contiguous(memory_format=cl)), keep(f"rb{i}.{j}.deq", (s_in * s_w).contiguous()),
+                              self.blocks[i][j - 1][2]))
+            self.qblocks.append(tuple(convs))
+
+    def _tower_fp8(self, x, xq, count=None):
+        """The residual tower on e4m3 K9: conv1 reads xq_l and writes yq_l only; conv2 reads yq_l and the bf16 skip x_l and
+        writes x_{l+1} over x_l plus (except in the last block) xq_{l+1} over xq_l."""
+        yq = torch.empty_like(xq, memory_format=torch.channels_last)
+        last = len(self.qblocks) - 1
+        for i, (c1, c2) in enumerate(self.qblocks):
+            _lib.conv3x3_c256_e4m3(xq, *c1, y=False, out_q=yq, inv_s_out=self._inv_sy[i:i + 1], count=count)
+            _lib.conv3x3_c256_e4m3(yq, *c2, skip=x, out=x, out_q=None if i == last else xq,
+                                   inv_s_out=None if i == last else self._inv_sx[i + 1:i + 2], count=count)
+        return x
 
     def _k9(self, x, w, b32, skip, out, count=None):
         if self.conv_events is None:
@@ -301,16 +414,24 @@ class BatchedEvaluator:
                 boards = uniq
             else:
                 self._n_unique_host += g
-            x = _lib.stem_lookup(boards, *self.stem_lookup, count=count)
+            if self.precision == "fp8":
+                x, xq = _lib.stem_lookup_e4m3(boards, *self.stem_lookup, self._inv_sx[0:1], count=count)
+            else:
+                x = _lib.stem_lookup(boards, *self.stem_lookup, count=count)
         else:
             g = planes.shape[0]
             x = planes.view(g, PLAYS * PIECES, 10, 9).contiguous(memory_format=torch.channels_last)
             x = self._conv_relu(x, self.stem)
+            if self.precision == "fp8":
+                xq = e4m3_quantize(x, self._inv_sx[0:1])
             self._n_unique_host += g
-        k9_plain, k9_skip = self.conv_impl == "k9", self.conv_impl in ("k9", "k9_skip")
-        for c1, c2 in self.blocks:
-            y = self._conv_relu(x, c1, k9_plain, count)
-            x = self._conv_add_relu(y, c2, x, k9_skip, count)
+        if self.precision == "fp8":
+            x = self._tower_fp8(x, xq, count)
+        else:
+            k9_plain, k9_skip = self.conv_impl == "k9", self.conv_impl in ("k9", "k9_skip")
+            for c1, c2 in self.blocks:
+                y = self._conv_relu(x, c1, k9_plain, count)
+                x = self._conv_add_relu(y, c2, x, k9_skip, count)
         if self.device.type == "cuda":
             # 1x1 heads = a GEMM over the (g*90, C) NHWC pixel rows (a view of the channels_last activations)
             rows = x.permute(0, 2, 3, 1).reshape(g * 90, x.shape[1])
@@ -364,7 +485,8 @@ class PolicyValueNet:
         self._evaluator = None
 
     def evaluator(self, **kw) -> BatchedEvaluator:
-        """The lockstep-batch bf16 evaluator over the current weights (CUDA only, no fallback)."""
+        """The lockstep-batch evaluator over the current weights (CUDA only, no fallback); ``precision="fp8"`` for the
+        e4m3 tower (see :class:`BatchedEvaluator`)."""
         if self.device.type != "cuda":
             raise _lib.CczError("BatchedEvaluator needs a CUDA device; there is no CPU fallback")
         if self._evaluator is None:

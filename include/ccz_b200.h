@@ -290,6 +290,24 @@ int ccz_heads_pack_rows(const void *d_h, int n, const int32_t *d_rows, void *d_o
 int ccz_leaf_unique(const uint8_t *d_boards, int n, int32_t *d_rows, uint8_t *d_uniq_boards, int32_t *d_n_unique,
                     unsigned long long *d_unique_total, ccz_stream_t s);
 
+/* K9 with e4m3 operands (tcgen05 kind::f8f6f4, fp32 accumulation), the FP8 evaluator's tower convolution:
+ *   f = acc * d_dequant[co] + d_bias[co] (+ skip) -> ReLU,  acc = sum over taps and channels of xq * wq (e4m3 values)
+ *   d_y  (may be NULL) bf16 [n,10,9,256] NHWC = bf16(f);  d_yq (may be NULL) e4m3 [n,10,9,256] = satfinite(f * *d_inv_s_out)
+ * d_xq: e4m3 [n,10,9,256] NHWC; d_wq: e4m3 [256][3][3][256]; d_dequant, d_bias: fp32[256] (dequant = s_in * s_w[co]);
+ * d_skip: bf16 like d_y or NULL, may alias d_y; d_inv_s_out: fp32 scalar on the device, read by the kernel (a captured
+ * graph follows a refreshed scale).  At least one output; neither output may alias d_xq, d_yq may not alias d_y or
+ * d_skip; every pointer 16-byte aligned.  The buffers hold `capacity` boards; d_n_boards NULL = all of them, otherwise
+ * the first min(*d_n_boards, capacity) as ccz_conv3x3_c256_count (each board's output is independent of its row, the
+ * batch size and the work plan).  CTA pairs, channel-sliced tail round. */
+int ccz_conv3x3_c256_e4m3(const void *d_xq, const void *d_wq, const float *d_dequant, const float *d_bias, const void *d_skip,
+                          void *d_y, void *d_yq, const float *d_inv_s_out, int capacity, const int32_t *d_n_boards,
+                          ccz_stream_t s);
+
+/* K10 with an e4m3 copy of its output: d_y as ccz_stem_lookup, d_yq e4m3 [n,10,9,256] = satfinite(d_y * *d_inv_s_out)
+ * (the bf16 value, scaled in fp32).  d_n_boards NULL = all `capacity` boards, otherwise as ccz_stem_lookup_count. */
+int ccz_stem_lookup_e4m3(const uint8_t *d_boards, int capacity, const int32_t *d_n_boards, const void *d_table,
+                         const float *d_bias_turn, void *d_y, void *d_yq, const float *d_inv_s_out, ccz_stream_t s);
+
 #ifdef __cplusplus
 }
 #endif
