@@ -1,7 +1,8 @@
 """K9 (csrc/ccz_conv.cuh): the tcgen05 / TMA-im2col 3x3 convolution with the fused ResBlock epilogue
 (net.py:33-41 with eval-mode BN folded) against a plain fp32 torch reference of the same op, through the
-C ABI (ccz_conv3x3_c256).  Tolerance: the output is rounded to bf16 (relative 2^-9) after an fp32
-accumulation over K = 2304 bf16 products, so |err| <= 2^-8 * max|ref| + small accumulation-order noise."""
+C ABI (ccz_conv3x3_c256).  The ragged-batch parity test bounds every element on its own (fp64 reference,
+tests/test_forward_stages_gpu.elementwise_bound): fp32 accumulation over K = 2304 bf16 products, the fp32 epilogue and
+one bf16 rounding of the output."""
 import pytest
 import torch
 import torch.nn.functional as F
@@ -32,12 +33,14 @@ def _ref(x, w, bias, skip):
 def test_conv_matches_fp32_reference(n, variant, with_skip):
     from chinesechesszero_b200 import _lib
 
+    from tests.test_forward_stages_gpu import K_CONV, conv_reference, conv_y_ratio, gamma_f16
+
     x, skip, w, bias = _case(n, seed=n)
     sk = skip if with_skip else None
     y = _lib.conv3x3_c256(x, w, bias, sk, variant=variant)
-    ref = _ref(x, w, bias, sk)
-    tol = 2.0 ** -8 * ref.abs().max().item() + 1e-3
-    assert (y.float() - ref).abs().max().item() <= tol
+    # fp64 reference of the same operands, per-element bound: fp32 accumulation over K + fp32 epilogue + bf16 output
+    pre, wx, babs = conv_reference(x, w, bias, sk)
+    assert conv_y_ratio(y, pre, wx, babs, gamma_f16(K_CONV)) <= 1.0
     assert y.is_contiguous(memory_format=torch.channels_last)
 
 
