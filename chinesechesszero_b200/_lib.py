@@ -30,7 +30,7 @@ NODE_BYTES = 24  # ccz_node (16) + ccz_link (8)
 MAX_CHILDREN = 119  # most legal moves of any Xiangqi position
 POLICY_PROBS, POLICY_LOGITS = 0, 1
 DEDUP_MAX_BOARDS = 16384  # largest leaf batch ccz_leaf_unique takes
-CONV_VARIANT_1CTA, CONV_VARIANT_PAIR, CONV_VARIANT_2PAIRS, CONV_VARIANT_4PAIRS = 1, 2, 2 | 32, 2 | 64
+CONV_VARIANT_1CTA, CONV_VARIANT_PAIR, CONV_VARIANT_2PAIRS, CONV_VARIANT_4PAIRS, CONV_VARIANT_PIXEL = 1, 2, 2 | 32, 2 | 64, 128
 
 EXPORTS = (
     "ccz_version", "ccz_last_error", "ccz_init", "ccz_action_table", "ccz_set_order_policy", "ccz_get_order_policy",
@@ -39,7 +39,7 @@ EXPORTS = (
     "ccz_mcts_reserve", "ccz_mcts_migrate", "ccz_mcts_select",
     "ccz_mcts_expand_backup", "ccz_mcts_root_visits", "ccz_mcts_advance", "ccz_replay_pack", "ccz_conv3x3_c256", "ccz_conv3x3_plan", "ccz_stem_lookup",
     "ccz_heads_pack", "ccz_conv3x3_c256_count", "ccz_stem_lookup_count", "ccz_heads_pack_rows", "ccz_leaf_unique",
-    "ccz_conv3x3_c256_e4m3", "ccz_stem_lookup_e4m3",
+    "ccz_conv3x3_c256_e4m3", "ccz_stem_lookup_e4m3", "ccz_conv3x3_c256_e4m3_variant",
 )
 
 
@@ -130,6 +130,7 @@ def load() -> ctypes.CDLL:
     lib.ccz_leaf_unique.argtypes = [vp, i32, vp, vp, vp, vp, vp]
     lib.ccz_conv3x3_c256_e4m3.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, i32, vp, vp]
     lib.ccz_stem_lookup_e4m3.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp, vp]
+    lib.ccz_conv3x3_c256_e4m3_variant.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, i32, vp, i32, vp]
     for name in EXPORTS:
         if name not in ("ccz_last_error",):
             getattr(lib, name).restype = i32
@@ -410,8 +411,9 @@ def conv3x3_c256(x: torch.Tensor, w: torch.Tensor, bias: torch.Tensor, skip: tor
 
     ``x`` / ``skip`` / ``out``: bf16 ``(n,256,10,9)`` tensors in ``torch.channels_last`` memory
     format (= NHWC rows of 256 channels); ``w``: bf16 ``(256,256,3,3)`` channels_last; ``bias`` fp32 (256,).
-    ``variant`` 0 = the library default; other values select the tiling for measurements
-    (``CONV_VARIANT_*``: 1 single-CTA tiles, 2 CTA pairs, 34 / 66 clusters of 2 / 4 pairs sharing weight stages).
+    ``variant`` 0 = the library default = ``CONV_VARIANT_PIXEL`` (pixel tiles: one board pixel x 256 boards per CTA pair);
+    other values select tiles of consecutive pixels for measurements (``CONV_VARIANT_*``: 1 single-CTA tiles, 2 CTA
+    pairs, 34 / 66 clusters of 2 / 4 pairs sharing weight stages), with the same results.
     ``count``: int32 (1,) device tensor -- only the first ``count`` boards are convolved (``ccz_conv3x3_c256_count``);
     the later rows of ``out`` are left unspecified.
     """
@@ -428,7 +430,7 @@ def conv3x3_c256(x: torch.Tensor, w: torch.Tensor, bias: torch.Tensor, skip: tor
         out = torch.empty_like(x, memory_format=cl)
     elif out.shape != x.shape or out.dtype != x.dtype or not out.is_contiguous(memory_format=cl):
         raise CczError("conv3x3_c256: out must match x (bf16, channels_last)")
-    if not 0 <= variant < 128:
+    if not 0 <= variant <= CONV_VARIANT_PIXEL:
         raise CczError("conv3x3_c256: variant out of range (see ccz_conv3x3_c256 in include/ccz_b200.h)")
     if not (x.is_cuda and w.is_cuda and bias.is_cuda and out.is_cuda):
         raise CczError("device tensor expected (the C ABI takes device pointers)")
@@ -462,13 +464,15 @@ def _check_scalar(name: str, what: str, t: torch.Tensor, dev) -> None:
 
 def conv3x3_c256_e4m3(xq: torch.Tensor, wq: torch.Tensor, dequant: torch.Tensor, bias: torch.Tensor, skip: torch.Tensor | None = None,
                       out: torch.Tensor | None = None, out_q: torch.Tensor | None = None, inv_s_out: torch.Tensor | None = None,
-                      y: bool = True, count: torch.Tensor | None = None):
+                      y: bool = True, count: torch.Tensor | None = None, variant: int = 0):
     """K9 with e4m3 operands: ``f = relu(conv3x3_pad1(xq, wq) * dequant + bias [+ skip])`` on the tcgen05 tensor cores.
 
     ``xq`` e4m3 ``(n,256,10,9)`` channels_last; ``wq`` e4m3 ``(256,256,3,3)`` channels_last; ``dequant`` / ``bias`` fp32
     (256,) (dequant[co] = input scale x weight scale of co); ``skip`` bf16 like ``xq`` (may be ``out``).  Outputs: the bf16
     ``out`` = bf16(f) when ``y`` (allocated unless given) and, when ``inv_s_out`` (fp32 (1,) device tensor) is given, the
     e4m3 ``out_q`` = satfinite(f * inv_s_out) (allocated unless given).  ``count`` as in :func:`conv3x3_c256`.
+    ``variant`` 0 = the default = ``CONV_VARIANT_PAIR`` (tiles of consecutive pixels), ``CONV_VARIANT_PIXEL`` = pixel
+    tiles (same results, slower in e4m3).
     Returns ``(out or None, out_q or None)``."""
     name = "conv3x3_c256_e4m3"
     _check_nhwc(name, "xq", xq, E4M3)
@@ -498,9 +502,10 @@ def conv3x3_c256_e4m3(xq: torch.Tensor, wq: torch.Tensor, dequant: torch.Tensor,
     if count is not None:
         _check_count(count, xq.device)
     with torch.cuda.device(xq.device):
-        check(load().ccz_conv3x3_c256_e4m3(xq.data_ptr(), wq.data_ptr(), dequant.data_ptr(), bias.data_ptr(), _ptr_or_none(skip),
-                                           _ptr_or_none(out), _ptr_or_none(out_q), _ptr_or_none(inv_s_out), n, _ptr_or_none(count),
-                                           stream_ptr(xq.device)), "ccz_conv3x3_c256_e4m3")
+        check(load().ccz_conv3x3_c256_e4m3_variant(xq.data_ptr(), wq.data_ptr(), dequant.data_ptr(), bias.data_ptr(),
+                                                   _ptr_or_none(skip), _ptr_or_none(out), _ptr_or_none(out_q), _ptr_or_none(inv_s_out),
+                                                   n, _ptr_or_none(count), int(variant), stream_ptr(xq.device)),
+              "ccz_conv3x3_c256_e4m3")
     return out, out_q
 
 

@@ -18,10 +18,6 @@
 #include "ccz_heads.cuh"
 #include "ccz_dedup.cuh"
 
-#ifndef CCZ_CONV_DEFAULT_PAIRS
-#define CCZ_CONV_DEFAULT_PAIRS 1
-#endif
-
 namespace {
 
 thread_local std::string g_err;
@@ -465,16 +461,18 @@ int conv3x3_c256_impl(const char *name, const void *d_x, const void *d_w, const 
     if (n_boards == 0) return 0;
     if (!d_x || !d_w || !d_bias || !d_y) return bad(-1, "NULL pointer");
     if (d_y == d_x) return bad(-1, "output must not alias the input (halo reads)");
-    if (variant < 0 || variant >= 128) return bad(-1, "bad variant");
-    // variant: 0 = default.  bits 0-1 CTA group (1 / 2), bit 2 = no tail split, bits 3-4 = traffic experiment
-    // (skips loads, WRONG results), bits 5-6 = log2(CTA pairs per cluster sharing a weight stage)
+    if (variant < 0 || variant > 128) return bad(-1, "bad variant");
+    // variant: 0 = default = 128 = pixel tiles on CTA pairs.  Otherwise tiles of consecutive pixels: bits 0-1 CTA group
+    // (1 / 2), bit 2 = no tail split, bits 3-4 = traffic experiment (skips loads, WRONG results), bits 5-6 = log2(CTA
+    // pairs per cluster sharing a weight stage)
+    const bool pix = variant == 0 || variant == 128;
+    if (pix) variant = 0;
     int cta_group = variant & 3;
     const int tail_split = !(variant & 4), dbg = (variant >> 3) & 3;
     int pairs = 1 << ((variant >> 5) & 3);
 #ifndef CCZ_CONV_EXPERIMENTS
     if (dbg) return bad(-1, "the load-skipping measurement variants need a -DCCZ_CONV_EXPERIMENTS build");
 #endif
-    if (variant == 0) { cta_group = 2; pairs = CCZ_CONV_DEFAULT_PAIRS; }
     if (cta_group == 0) cta_group = 2;
     if (cta_group == 3 || pairs > 4 || (cta_group == 1 && pairs != 1))
         return bad(-1, "unsupported variant (cta_group 1|2, pairs 1|2|4, pairs > 1 needs cta_group 2)");
@@ -483,39 +481,48 @@ int conv3x3_c256_impl(const char *name, const void *d_x, const void *d_w, const 
     static cv::Driver drv;
     if (const char *err = cv::driver_init(drv)) return fail(-3, err);
     const long long m = (long long)n_boards * cv::BOARD_HW;
-    const int rows_per_tile = cv::BM * cta_group * pairs;
-    const int n_tiles = (int)((m + rows_per_tile - 1) / rows_per_tile);
+    const int n_units = cv::conv_units(n_boards, pix, cv::BM * cta_group * pairs);
     CUtensorMap tx, tw, ts, ty;
-    if (!cv::encode_im2col(drv, &tx, d_x, n_boards)) return bad(-3, "cuTensorMapEncodeIm2col(x) failed");
+    if (pix ? !cv::encode_pixels(drv, &tx, d_x, n_boards) : !cv::encode_im2col(drv, &tx, d_x, n_boards))
+        return bad(-3, "cuTensorMapEncode(x) failed");
     if (!cv::encode_rows(drv, &tw, d_w, cv::BN, 9 * cv::C, (uint32_t)(cv::BN / cta_group / pairs)))
         return bad(-3, "cuTensorMapEncodeTiled(w) failed");
-    if (!cv::encode_rows(drv, &ty, d_y, (uint64_t)m, cv::C, cv::BM)) return bad(-3, "cuTensorMapEncodeTiled(y) failed");
+    auto encode_out = [&](CUtensorMap *t, const void *p) {
+        return pix ? cv::encode_pixels(drv, t, p, n_boards) : cv::encode_rows(drv, t, p, (uint64_t)m, cv::C, cv::BM);
+    };
+    if (!encode_out(&ty, d_y)) return bad(-3, "cuTensorMapEncodeTiled(y) failed");
     if (d_skip) {
-        if (!cv::encode_rows(drv, &ts, d_skip, (uint64_t)m, cv::C, cv::BM)) return bad(-3, "cuTensorMapEncodeTiled(skip) failed");
+        if (!encode_out(&ts, d_skip)) return bad(-3, "cuTensorMapEncodeTiled(skip) failed");
     } else {
         ts = ty;
     }
     cudaError_t e;
-#define CCZ_CONV_LAUNCH_C(CG, PAIRS, CNT)                                                                                  \
-    (d_skip ? cv::launch_variant<CG, PAIRS, true, CNT>(tx, tw, ts, ty, d_bias, n_tiles, tail_split, dbg, d_count, n_boards, s) \
-            : cv::launch_variant<CG, PAIRS, false, CNT>(tx, tw, ts, ty, d_bias, n_tiles, tail_split, dbg, d_count, n_boards, s))
-#define CCZ_CONV_LAUNCH(CG, PAIRS) (d_count ? CCZ_CONV_LAUNCH_C(CG, PAIRS, true) : CCZ_CONV_LAUNCH_C(CG, PAIRS, false))
-    if (cta_group == 1) e = CCZ_CONV_LAUNCH(1, 1);
-    else if (pairs == 1) e = CCZ_CONV_LAUNCH(2, 1);
-    else if (pairs == 2) e = CCZ_CONV_LAUNCH(2, 2);
-    else e = CCZ_CONV_LAUNCH(2, 4);
+#define CCZ_CONV_LAUNCH_C(CG, PAIRS, CNT, PIX)                                                                                              \
+    (d_skip ? cv::launch_variant<CG, PAIRS, true, CNT, __nv_bfloat16, PIX>(tx, tw, ts, ty, d_bias, n_units, tail_split, dbg, d_count, n_boards, s) \
+            : cv::launch_variant<CG, PAIRS, false, CNT, __nv_bfloat16, PIX>(tx, tw, ts, ty, d_bias, n_units, tail_split, dbg, d_count, n_boards, s))
+#define CCZ_CONV_LAUNCH(CG, PAIRS, PIX) (d_count ? CCZ_CONV_LAUNCH_C(CG, PAIRS, true, PIX) : CCZ_CONV_LAUNCH_C(CG, PAIRS, false, PIX))
+    if (pix) e = CCZ_CONV_LAUNCH(2, 1, true);
+    else if (cta_group == 1) e = CCZ_CONV_LAUNCH(1, 1, false);
+    else if (pairs == 1) e = CCZ_CONV_LAUNCH(2, 1, false);
+    else if (pairs == 2) e = CCZ_CONV_LAUNCH(2, 2, false);
+    else e = CCZ_CONV_LAUNCH(2, 4, false);
 #undef CCZ_CONV_LAUNCH
 #undef CCZ_CONV_LAUNCH_C
     if (e != cudaSuccess) return fail(-2, "conv3x3_c256_kernel launch", e);
     return 0;
 }
 
-// e4m3 tower convolution: always CTA pairs (cta_group::2), one pair per cluster, tail split on.
+// e4m3 tower convolution: always CTA pairs (cta_group::2), one pair per cluster, tail split on; variant 0 = default = 2 =
+// tiles of consecutive pixels, 128 = pixel tiles (slower for e4m3, whose main loop is too short to hide the epilogue of
+// the 8- and 12-k-block border tiles; DESIGN.md "K9 in detail").
 int conv3x3_c256_e4m3_impl(const void *d_xq, const void *d_wq, const float *d_dequant, const float *d_bias, const void *d_skip, void *d_y,
-                           void *d_yq, const float *d_inv_s_out, int n_boards, const int32_t *d_count, ccz_stream_t s) {
+                           void *d_yq, const float *d_inv_s_out, int n_boards, const int32_t *d_count, int variant, ccz_stream_t s) {
     namespace cv = ccz::conv;
     using E = __nv_fp8_e4m3;
     auto bad = [&](int code, const char *what) { return fail(code, (std::string("ccz_conv3x3_c256_e4m3: ") + what).c_str()); };
+    if (variant != 0 && variant != 2 && variant != 128)
+        return bad(-1, "variant must be 0 (default), 2 (tiles of consecutive pixels) or 128 (pixel tiles)");
+    const bool pix = variant == 128;
     if (n_boards < 0) return bad(-1, "capacity < 0");
     if (n_boards == 0) return 0;
     if (!d_xq || !d_wq || !d_dequant || !d_bias) return bad(-1, "NULL pointer");
@@ -529,16 +536,19 @@ int conv3x3_c256_e4m3_impl(const void *d_xq, const void *d_wq, const float *d_de
     static cv::Driver drv;
     if (const char *err = cv::driver_init(drv)) return fail(-3, err);
     const long long m = (long long)n_boards * cv::BOARD_HW;
-    const int rows_per_tile = cv::BM * 2;
-    const int n_tiles = (int)((m + rows_per_tile - 1) / rows_per_tile);
+    const int n_units = cv::conv_units(n_boards, pix, cv::BM * 2);
     CUtensorMap tx, tw, ts, ty;
-    if (!cv::encode_im2col(drv, &tx, d_xq, n_boards, true)) return bad(-3, "cuTensorMapEncodeIm2col(xq) failed");
+    if (pix ? !cv::encode_pixels(drv, &tx, d_xq, n_boards, true) : !cv::encode_im2col(drv, &tx, d_xq, n_boards, true))
+        return bad(-3, "cuTensorMapEncode(xq) failed");
     if (!cv::encode_rows(drv, &tw, d_wq, cv::BN, 9 * cv::C, (uint32_t)(cv::BN / 2), true)) return bad(-3, "cuTensorMapEncodeTiled(wq) failed");
+    auto encode_out = [&](CUtensorMap *t, const void *p, bool e4m3) {
+        return pix ? cv::encode_pixels(drv, t, p, n_boards, e4m3) : cv::encode_rows(drv, t, p, (uint64_t)m, cv::C, cv::BM, e4m3);
+    };
     // without a bf16 output the y map is encoded over the skip (or the input) and never stored through
     const void *y_map = d_y ? d_y : (d_skip ? d_skip : d_xq);
-    if (!cv::encode_rows(drv, &ty, y_map, (uint64_t)m, cv::C, cv::BM, !d_y && !d_skip)) return bad(-3, "cuTensorMapEncodeTiled(y) failed");
+    if (!encode_out(&ty, y_map, !d_y && !d_skip)) return bad(-3, "cuTensorMapEncodeTiled(y) failed");
     if (d_skip) {
-        if (!cv::encode_rows(drv, &ts, d_skip, (uint64_t)m, cv::C, cv::BM)) return bad(-3, "cuTensorMapEncodeTiled(skip) failed");
+        if (!encode_out(&ts, d_skip, false)) return bad(-3, "cuTensorMapEncodeTiled(skip) failed");
     } else {
         ts = ty;
     }
@@ -549,12 +559,12 @@ int conv3x3_c256_e4m3_impl(const void *d_xq, const void *d_wq, const float *d_de
     qo.rows = m;
     qo.out_y = d_y != nullptr;
     cudaError_t e;
-    if (d_count)
-        e = d_skip ? cv::launch_variant<2, 1, true, true, E>(tx, tw, ts, ty, d_bias, n_tiles, 1, 0, d_count, n_boards, s, qo)
-                   : cv::launch_variant<2, 1, false, true, E>(tx, tw, ts, ty, d_bias, n_tiles, 1, 0, d_count, n_boards, s, qo);
-    else
-        e = d_skip ? cv::launch_variant<2, 1, true, false, E>(tx, tw, ts, ty, d_bias, n_tiles, 1, 0, nullptr, n_boards, s, qo)
-                   : cv::launch_variant<2, 1, false, false, E>(tx, tw, ts, ty, d_bias, n_tiles, 1, 0, nullptr, n_boards, s, qo);
+#define CCZ_CONV_LAUNCH_Q(CNT, PIX)                                                                                          \
+    (d_skip ? cv::launch_variant<2, 1, true, CNT, E, PIX>(tx, tw, ts, ty, d_bias, n_units, 1, 0, d_count, n_boards, s, qo) \
+            : cv::launch_variant<2, 1, false, CNT, E, PIX>(tx, tw, ts, ty, d_bias, n_units, 1, 0, d_count, n_boards, s, qo))
+    if (d_count) e = pix ? CCZ_CONV_LAUNCH_Q(true, true) : CCZ_CONV_LAUNCH_Q(true, false);
+    else e = pix ? CCZ_CONV_LAUNCH_Q(false, true) : CCZ_CONV_LAUNCH_Q(false, false);
+#undef CCZ_CONV_LAUNCH_Q
     if (e != cudaSuccess) return fail(-2, "conv3x3_c256_kernel<e4m3> launch", e);
     return 0;
 }
@@ -635,7 +645,6 @@ int ccz_conv3x3_plan(int n_boards, int variant, int resident_clusters, int32_t *
     if (n_boards <= 0 || resident_clusters <= 0 || !out || variant < 0 || variant >= 128)
         return fail(-1, "ccz_conv3x3_plan: bad argument");
     int cta_group = variant & 3, pairs = 1 << ((variant >> 5) & 3);
-    if (variant == 0) { cta_group = 2; pairs = CCZ_CONV_DEFAULT_PAIRS; }
     if (cta_group == 0) cta_group = 2;
     if (cta_group == 3 || pairs > 4 || (cta_group == 1 && pairs != 1)) return fail(-1, "ccz_conv3x3_plan: unsupported variant");
     const long long m = (long long)n_boards * cv::BOARD_HW;
@@ -658,8 +667,15 @@ int ccz_stem_lookup_count(const uint8_t *d_boards, int capacity, const int32_t *
 
 int ccz_conv3x3_c256_e4m3(const void *d_xq, const void *d_wq, const float *d_dequant, const float *d_bias, const void *d_skip, void *d_y,
                           void *d_yq, const float *d_inv_s_out, int capacity, const int32_t *d_n_boards, ccz_stream_t s) {
-    return conv3x3_c256_e4m3_impl(d_xq, d_wq, d_dequant, d_bias, d_skip, d_y, d_yq, d_inv_s_out, capacity, d_n_boards, s);
+    return conv3x3_c256_e4m3_impl(d_xq, d_wq, d_dequant, d_bias, d_skip, d_y, d_yq, d_inv_s_out, capacity, d_n_boards, 0, s);
 }
+
+int ccz_conv3x3_c256_e4m3_variant(const void *d_xq, const void *d_wq, const float *d_dequant, const float *d_bias, const void *d_skip,
+                                  void *d_y, void *d_yq, const float *d_inv_s_out, int capacity, const int32_t *d_n_boards, int variant,
+                                  ccz_stream_t s) {
+    return conv3x3_c256_e4m3_impl(d_xq, d_wq, d_dequant, d_bias, d_skip, d_y, d_yq, d_inv_s_out, capacity, d_n_boards, variant, s);
+}
+
 
 int ccz_stem_lookup_e4m3(const uint8_t *d_boards, int capacity, const int32_t *d_n_boards, const void *d_table, const float *d_bias_turn,
                          void *d_y, void *d_yq, const float *d_inv_s_out, ccz_stream_t s) {

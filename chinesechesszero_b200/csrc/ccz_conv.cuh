@@ -5,9 +5,11 @@
 //   D[m, co] = relu( sum_{tap, ci} X[pixel(m) + tap, ci] * Wt[co, tap, ci] + bias[co] (+ skip[m, co]) )
 //
 // m runs over the n*90 output pixels (NHWC, channel-contiguous), K = 9 taps x 256 channels = 2304.
-//   * A operand (activations): TMA *im2col* loads, 128 pixels x 64 channels per stage, 128-byte swizzle;
-//     the TMA unit walks w, h, n in output-pixel order and zero-fills the halo, so an M tile is any
-//     128 consecutive pixels and no FLOP is spent on padding.
+//   * A operand (activations), 128 rows x 64 channels per stage, 128-byte swizzle, in one of two tilings:
+//     - pixel tiles (PIX, the bf16 default): the rows are one board pixel of 128 consecutive boards, loaded by a plain
+//       3-D tiled TMA; only the taps that fall on the board are loaded and multiplied (see "pixel tiles" below).
+//     - consecutive pixels: TMA *im2col* loads; the TMA unit walks w, h, n in output-pixel order and zero-fills the
+//       halo, so an M tile is any 128 consecutive pixels, and the zero products of the halo are multiplied.
 //   * B operand (weights, [256][9*256] K-major): plain 2-D tiled TMA, same swizzle.
 //   * MMA: tcgen05.mma kind::f16 (bf16 in, fp32 accumulate in TMEM), issued by one thread.  CG = 2 pairs
 //     two CTAs of a cluster on one 256x256 tile (cta_group::2): each CTA stages its own 128 pixel rows
@@ -206,6 +208,26 @@ __device__ __forceinline__ void tma_load_im2col(uint32_t dst, const CUtensorMap 
             : "memory");
     }
 }
+// 3-D tiled load over the (c, pixel, board) view of the activations.  CG == 2: as tma_load_2d.
+template <int CG>
+__device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap *m, uint32_t bar, int c0, int c1, int c2) {
+    if constexpr (CG == 1) {
+        asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(dst),
+                     "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2)
+                     : "memory");
+    } else {
+        asm volatile(
+            "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4, %5}], "
+            "[%2], %6;" ::"r"(dst),
+            "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "l"(L2_HINT_DEFAULT)
+            : "memory");
+    }
+}
+__device__ __forceinline__ void tma_store_3d(const CUtensorMap *m, uint32_t src, int c0, int c1, int c2) {
+    asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];" ::"l"(reinterpret_cast<uint64_t>(m)),
+                 "r"(src), "r"(c0), "r"(c1), "r"(c2)
+                 : "memory");
+}
 __device__ __forceinline__ void tma_store_2d(const CUtensorMap *m, uint32_t src, int c0, int c1) {
     asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(reinterpret_cast<uint64_t>(m)), "r"(src),
                  "r"(c0), "r"(c1)
@@ -365,6 +387,81 @@ __host__ __device__ inline Plan plan_items(int n_tiles, int clusters, bool tail_
     return p;
 }
 
+// ---- pixel tiles (the default mapping) ----------------------------------------------------------
+// A pixel tile is one board pixel P of a block of BM * CG boards: CTA r of the pair holds boards blk * BM * CG + r * BM + i
+// at P in its row i.  Every row of the tile then has the same in-board filter taps, so only those taps are loaded and
+// multiplied: 4 of 9 at the 4 corners, 6 at the 30 edge pixels, 9 at the 56 interior ones, 700 of the 810 (pixel, tap)
+// pairs of a board.  The zero-padding products that a tile of consecutive pixels has to multiply are never issued.
+//
+// Tiles are scheduled in BUNDLES of equal cost, 39 per board block: 28 pairs of vertically adjacent interior pixels and
+// 10 runs of 3 edge pixels along the border (18 taps each), and the 4 corners (16 taps).  Bundles then go through
+// plan_items exactly as consecutive-pixel tiles do (round-robin, channel-sliced last round), which balances the clusters
+// without a cost model, and block-major bundle order keeps the clusters on the same one or two board blocks (12 MB of
+// bf16 input each) so that the 9 reads of every input pixel hit L2.
+constexpr int BUNDLES = 39;
+__host__ __device__ inline int bundle_first(int k) { return k < 28 ? 2 * k : k < 38 ? 56 + 3 * (k - 28) : 86; }
+__host__ __device__ inline int bundle_size(int k) { return k < 28 ? 2 : k < 38 ? 3 : 4; }
+// board pixel (h * 9 + w) of position i of the bundle order: interior pixels in vertical pairs, then the 30 edge pixels
+// clockwise from (0,1), then the corners
+__host__ __device__ inline int bundle_pixel(int i) {
+    int h, w;
+    if (i < 56) {
+        const int j = i >> 1;
+        h = 1 + 2 * (j / 7) + (i & 1);
+        w = 1 + j % 7;
+    } else if (i < 86) {
+        const int e = i - 56;
+        if (e < 7) { h = 0; w = 1 + e; }
+        else if (e < 15) { h = 1 + (e - 7); w = 8; }
+        else if (e < 22) { h = 9; w = 7 - (e - 15); }
+        else { h = 8 - (e - 22); w = 0; }
+    } else {
+        const int c = i - 86;
+        h = c < 2 ? 0 : 9;
+        w = (c == 1 || c == 2) ? 8 : 0;
+    }
+    return h * BOARD_W + w;
+}
+// bit tap (= kh * 3 + kw) set when input pixel (h + kh - 1, w + kw - 1) lies on the board
+__host__ __device__ inline uint32_t pixel_taps(int pix) {
+    const int h = pix / BOARD_W, w = pix - h * BOARD_W;
+    const uint32_t cols = (w == 0 ? 6u : w == BOARD_W - 1 ? 3u : 7u), rows = (h == 0 ? 6u : h == BOARD_H - 1 ? 3u : 7u);
+    uint32_t m = 0;
+    for (int r = 0; r < 3; ++r)
+        if (rows >> r & 1) m |= cols << (3 * r);
+    return m;
+}
+// scheduling units of one launch over n_boards boards, with rows = BM * CTAs per cluster: bundles of pixel tiles over
+// blocks of `rows` boards, or cluster tiles of `rows` consecutive pixels
+__host__ __device__ inline int conv_units(int n_boards, bool pix, int rows) {
+    return pix ? BUNDLES * ((n_boards + rows - 1) / rows) : (int)(((long long)n_boards * BOARD_HW + rows - 1) / rows);
+}
+
+// Output rows of one CTA in tile `sub` of work unit `unit`.  PIX: board pixel `pix` of boards b0 .. b0 + BM - 1, and the
+// in-board taps of that pixel; otherwise the BM consecutive NHWC pixel rows from m0, all taps.
+struct TileRows {
+    int m0, pix, b0;
+    uint32_t taps;
+};
+template <int CG, int PAIRS, bool PIX>
+__device__ __forceinline__ TileRows tile_rows(int unit, int sub, uint32_t pair_id, uint32_t prank) {
+    TileRows t{0, 0, 0, 0x1FFu};
+    if constexpr (PIX) {
+        const int blk = unit / BUNDLES;
+        t.pix = bundle_pixel(bundle_first(unit - blk * BUNDLES) + sub);
+        t.b0 = (blk * CG + (int)prank) * BM;
+        t.taps = pixel_taps(t.pix);
+    } else {
+        t.m0 = ((unit * PAIRS + (int)pair_id) * CG + (int)prank) * BM;
+    }
+    return t;
+}
+template <bool PIX>
+__device__ __forceinline__ int unit_tiles(int unit) {
+    if constexpr (PIX) return bundle_size(unit % BUNDLES);
+    return 1;
+}
+
 // PAIRS > 1 (CG == 2 only): a cluster of PAIRS CTA pairs works on PAIRS consecutive tiles with the SAME weight
 // stage: each CTA fetches 1/PAIRS of its half of the weight tile and multicasts it to the CTAs of equal
 // parity, so weight traffic from L2 drops by PAIRS.  A stage is then free only when every pair has consumed it.
@@ -374,13 +471,18 @@ __host__ __device__ inline Plan plan_items(int n_tiles, int clusters, bool tail_
 // the clusters without an item only allocate / free TMEM and pass the cluster barriers.
 //
 // T = __nv_fp8_e4m3: x and w are e4m3, the accumulator is dequantised per output channel in the epilogue (QOut).
-template <int CG, int PAIRS, bool HAS_SKIP, bool DEV_COUNT, typename T = __nv_bfloat16>
+//
+// PIX: pixel tiles.  A work item's unit is a bundle of pixel tiles, run one after the other; x, skip and y are (c, pixel,
+// board) tensor maps with 128-board boxes, and each tile loads and multiplies only the k-blocks of its in-board taps, in
+// the same order as a consecutive-pixel tile (a dropped k-block only adds exact zeros to every accumulator of the tile).
+template <int CG, int PAIRS, bool HAS_SKIP, bool DEV_COUNT, typename T = __nv_bfloat16, bool PIX = false>
 __global__ void __launch_bounds__(THREADS, 1)
 conv3x3_c256_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUtensorMap tm_w,
                     const __grid_constant__ CUtensorMap tm_skip, const __grid_constant__ CUtensorMap tm_y, const float *__restrict__ bias,
                     int n_items, int n_full, int split_log2, int dbg, const int32_t *__restrict__ d_count, int count_cap, int tail_split,
                     const QOut<T> qo) {
     using K = Cfg<CG, T>;
+    static_assert(!PIX || PAIRS == 1, "pixel tiles run on single CTA pairs");
     extern __shared__ uint8_t smem_raw[];
     const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
     const uint32_t a_smem = smem_base;
@@ -405,8 +507,8 @@ conv3x3_c256_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
     const uint32_t prank = rank % CG, pair_id = rank / CG, lead_rank = rank - prank; // position in the pair / pair in the cluster
     const int cluster_id = blockIdx.x / CLUSTER, n_clusters = gridDim.x / CLUSTER;
     if constexpr (DEV_COUNT) {
-        const int nb = min(max(*d_count, 0), count_cap), rows_per_tile = BM * CLUSTER;
-        const Plan pl = plan_items((nb * BOARD_HW + rows_per_tile - 1) / rows_per_tile, n_clusters, tail_split != 0);
+        const int nb = min(max(*d_count, 0), count_cap);
+        const Plan pl = plan_items(conv_units(nb, PIX, BM * CLUSTER), n_clusters, tail_split != 0);
         n_items = pl.n_items;
         n_full = pl.n_full;
         split_log2 = pl.split_log2;
@@ -457,24 +559,33 @@ conv3x3_c256_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
             uint32_t phase = 0;
             for (int item = cluster_id; item < n_items; item += n_clusters) {
                 const WorkItem wi = work_item(item, n_full, split_log2);
-                const int m0 = ((wi.tile * PAIRS + (int)pair_id) * CG + (int)prank) * BM;
                 const int b_row = wi.n_off + (int)prank * (wi.n_w / CG); // a channel slice over-reads rows it does not use
-                const int img = m0 / BOARD_HW, rem = m0 - img * BOARD_HW;
-                const int p = rem / BOARD_W, q = rem - p * BOARD_W;
-                for (int kb = 0; kb < K::KBLOCKS; ++kb) {
-                    const int tap = kb >> K::CBLK_LOG2, c0 = (kb & ((1 << K::CBLK_LOG2) - 1)) * K::BK;
-                    const int r = tap / 3, s = tap - 3 * r;
-                    mbar_wait(bar_empty + 8 * stage, phase ^ 1);
-                    const bool do_a = !((dbg & 2) && (kb & 1)), do_b = !((dbg & 1) && (kb & 1)); // traffic-sensitivity experiment
-                    if (prank == 0) mbar_expect_tx(bar_full + 8 * stage, CG * ((do_a ? K::A_BYTES : 0) + (do_b ? K::B_BYTES : 0)));
-                    if (do_a) tma_load_im2col<CG>(a_smem + stage * K::A_BYTES, &tm_x, full0 + 8 * stage, c0, q - 1, p - 1, img, (uint16_t)s, (uint16_t)r);
-                    if constexpr (PAIRS == 1) {
-                        if (do_b) tma_load_2d<CG>(b_smem + stage * K::B_BYTES, &tm_w, full0 + 8 * stage, kb * K::BK, b_row);
-                    } else {
-                        tma_load_2d_mc(b_smem + stage * K::B_BYTES + (int)pair_id * SLICE_ROWS * 128, &tm_w, full0 + 8 * stage, kb * K::BK,
-                                       b_row + (int)pair_id * SLICE_ROWS, mc_mask);
+                for (int sub = 0; sub < unit_tiles<PIX>(wi.tile); ++sub) {
+                    const TileRows tr = tile_rows<CG, PAIRS, PIX>(wi.tile, sub, pair_id, prank);
+                    const int img = tr.m0 / BOARD_HW, rem = tr.m0 - img * BOARD_HW;
+                    const int p = rem / BOARD_W, q = rem - p * BOARD_W;
+                    for (int kb = 0; kb < K::KBLOCKS; ++kb) {
+                        const int tap = kb >> K::CBLK_LOG2, c0 = (kb & ((1 << K::CBLK_LOG2) - 1)) * K::BK;
+                        if (!(tr.taps >> tap & 1u)) continue;
+                        const int r = tap / 3, s = tap - 3 * r;
+                        mbar_wait(bar_empty + 8 * stage, phase ^ 1);
+                        const bool do_a = !((dbg & 2) && (kb & 1)), do_b = !((dbg & 1) && (kb & 1)); // traffic-sensitivity experiment
+                        if (prank == 0) mbar_expect_tx(bar_full + 8 * stage, CG * ((do_a ? K::A_BYTES : 0) + (do_b ? K::B_BYTES : 0)));
+                        if (do_a) {
+                            if constexpr (PIX)
+                                tma_load_3d<CG>(a_smem + stage * K::A_BYTES, &tm_x, full0 + 8 * stage, c0, tr.pix + (r - 1) * BOARD_W + (s - 1), tr.b0);
+                            else
+                                tma_load_im2col<CG>(a_smem + stage * K::A_BYTES, &tm_x, full0 + 8 * stage, c0, q - 1, p - 1, img, (uint16_t)s,
+                                                    (uint16_t)r);
+                        }
+                        if constexpr (PAIRS == 1) {
+                            if (do_b) tma_load_2d<CG>(b_smem + stage * K::B_BYTES, &tm_w, full0 + 8 * stage, kb * K::BK, b_row);
+                        } else {
+                            tma_load_2d_mc(b_smem + stage * K::B_BYTES + (int)pair_id * SLICE_ROWS * 128, &tm_w, full0 + 8 * stage, kb * K::BK,
+                                           b_row + (int)pair_id * SLICE_ROWS, mc_mask);
+                        }
+                        if (++stage == K::STAGES) { stage = 0; phase ^= 1; }
                     }
-                    if (++stage == K::STAGES) { stage = 0; phase ^= 1; }
                 }
             }
         }
@@ -486,39 +597,53 @@ conv3x3_c256_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
             int stage = 0;
             uint32_t phase = 0, acc = 0, acc_phase = 0;
             for (int item = cluster_id; item < n_items; item += n_clusters) {
-                const uint32_t idesc = umma_idesc(BM * CG, work_item(item, n_full, split_log2).n_w, K::FP8 ? 0u : 1u);
-                mbar_wait_cluster(bar_tempty + 8 * acc, acc_phase ^ 1);
-                tc_fence_after();
-                const uint32_t d_tmem = tmem_base + acc * BN;
-                for (int kb = 0; kb < K::KBLOCKS; ++kb) {
-                    mbar_wait(bar_full + 8 * stage, phase);
+                const WorkItem wi = work_item(item, n_full, split_log2);
+                const uint32_t idesc = umma_idesc(BM * CG, wi.n_w, K::FP8 ? 0u : 1u);
+                for (int sub = 0; sub < unit_tiles<PIX>(wi.tile); ++sub) {
+                    const uint32_t taps = tile_rows<CG, PAIRS, PIX>(wi.tile, sub, pair_id, prank).taps;
+                    mbar_wait_cluster(bar_tempty + 8 * acc, acc_phase ^ 1);
                     tc_fence_after();
-                    const uint64_t a_desc = umma_desc_sw128(a_smem + stage * K::A_BYTES);
-                    const uint64_t b_desc = umma_desc_sw128(b_smem + stage * K::B_BYTES);
+                    const uint32_t d_tmem = tmem_base + acc * BN;
+                    uint32_t started = 0; // the tile's first MMA overwrites the accumulator
+                    for (int kb = 0; kb < K::KBLOCKS; ++kb) {
+                        if (!(taps >> (kb >> K::CBLK_LOG2) & 1u)) continue;
+                        mbar_wait(bar_full + 8 * stage, phase);
+                        tc_fence_after();
+                        const uint64_t a_desc = umma_desc_sw128(a_smem + stage * K::A_BYTES);
+                        const uint64_t b_desc = umma_desc_sw128(b_smem + stage * K::B_BYTES);
 #pragma unroll
-                    for (int k = 0; k < K::BK / K::UMMA_K; ++k) { // +32 bytes along K inside the swizzle row
-                        if constexpr (K::FP8)
-                            umma_e4m3<CG>(d_tmem, a_desc + 2 * k, b_desc + 2 * k, idesc, (uint32_t)((kb | k) != 0));
-                        else
-                            umma_bf16<CG>(d_tmem, a_desc + 2 * k, b_desc + 2 * k, idesc, (uint32_t)((kb | k) != 0));
+                        for (int k = 0; k < K::BK / K::UMMA_K; ++k) { // +32 bytes along K inside the swizzle row
+                            if constexpr (K::FP8)
+                                umma_e4m3<CG>(d_tmem, a_desc + 2 * k, b_desc + 2 * k, idesc, started | (uint32_t)(k != 0));
+                            else
+                                umma_bf16<CG>(d_tmem, a_desc + 2 * k, b_desc + 2 * k, idesc, started | (uint32_t)(k != 0));
+                        }
+                        started = 1;
+                        umma_commit<CG>(bar_empty + 8 * stage, mask_cluster);
+                        if (++stage == K::STAGES) { stage = 0; phase ^= 1; }
                     }
-                    umma_commit<CG>(bar_empty + 8 * stage, mask_cluster);
-                    if (++stage == K::STAGES) { stage = 0; phase ^= 1; }
+                    umma_commit<CG>(bar_tfull + 8 * acc, mask_pair);
+                    if (++acc == 2) { acc = 0; acc_phase ^= 1; }
                 }
-                umma_commit<CG>(bar_tfull + 8 * acc, mask_pair);
-                if (++acc == 2) { acc = 0; acc_phase ^= 1; }
             }
         }
     } else if (warp == 3) {
         // ===== skip-tile producer: prefetch skip[m0 : m0+128, :] into the staging tile =====
         if (HAS_SKIP && lane == 0) {
             uint32_t it = 0;
-            for (int item = cluster_id; item < n_items; item += n_clusters, ++it) {
+            for (int item = cluster_id; item < n_items; item += n_clusters) {
                 const WorkItem wi = work_item(item, n_full, split_log2);
-                const int m0 = ((wi.tile * PAIRS + (int)pair_id) * CG + (int)prank) * BM;
-                mbar_wait_relaxed(bar_stfree, (it & 1) ^ 1);
-                mbar_expect_tx(bar_skip, (wi.n_w / 64) * (BM * 128));
-                for (int g = 0; g < wi.n_w / 64; ++g) tma_load_2d<1>(staging + g * (BM * 128), &tm_skip, bar_skip, wi.n_off + g * 64, m0);
+                for (int sub = 0; sub < unit_tiles<PIX>(wi.tile); ++sub, ++it) {
+                    const TileRows tr = tile_rows<CG, PAIRS, PIX>(wi.tile, sub, pair_id, prank);
+                    mbar_wait_relaxed(bar_stfree, (it & 1) ^ 1);
+                    mbar_expect_tx(bar_skip, (wi.n_w / 64) * (BM * 128));
+                    for (int g = 0; g < wi.n_w / 64; ++g) {
+                        if constexpr (PIX)
+                            tma_load_3d<1>(staging + g * (BM * 128), &tm_skip, bar_skip, wi.n_off + g * 64, tr.pix, tr.b0);
+                        else
+                            tma_load_2d<1>(staging + g * (BM * 128), &tm_skip, bar_skip, wi.n_off + g * 64, tr.m0);
+                    }
+                }
             }
         }
     } else if (warp >= 4) {
@@ -533,93 +658,102 @@ conv3x3_c256_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
             if (qo.yq) inv_s = *qo.inv_s_out;
         }
         uint32_t acc = 0, acc_phase = 0, it = 0;
-        for (int item = cluster_id; item < n_items; item += n_clusters, ++it) {
+        for (int item = cluster_id; item < n_items; item += n_clusters) {
             const WorkItem wi = work_item(item, n_full, split_log2);
-            const int m0 = ((wi.tile * PAIRS + (int)pair_id) * CG + (int)prank) * BM;
-            if (HAS_SKIP) mbar_wait_relaxed(bar_skip, it & 1);
-            mbar_wait_relaxed(bar_tfull + 8 * acc, acc_phase);
-            tc_fence_after();
-            const uint32_t t_row = tmem_base + ((uint32_t)(quarter * 32) << 16) + acc * BN;
+            for (int sub = 0; sub < unit_tiles<PIX>(wi.tile); ++sub, ++it) {
+                const TileRows tr = tile_rows<CG, PAIRS, PIX>(wi.tile, sub, pair_id, prank);
+                const long long q_row = PIX ? (long long)(tr.b0 + row) * BOARD_HW + tr.pix : (long long)tr.m0 + row; // e4m3 yq row
+                if (HAS_SKIP) mbar_wait_relaxed(bar_skip, it & 1);
+                mbar_wait_relaxed(bar_tfull + 8 * acc, acc_phase);
+                tc_fence_after();
+                const uint32_t t_row = tmem_base + ((uint32_t)(quarter * 32) << 16) + acc * BN;
 #pragma unroll 1
-            for (int chunk = 0; chunk < wi.n_w / 32; ++chunk) { // 32 channels per chunk
-                uint32_t v[32];
-                tmem_ld32(t_row + chunk * 32, v);
-                tmem_ld_wait();
-                uint8_t *box_row = stg + (chunk >> 1) * (BM * 128) + row * 128;
-                [[maybe_unused]] uint32_t q[8]; // e4m3: the chunk's 32 output bytes
+                for (int chunk = 0; chunk < wi.n_w / 32; ++chunk) { // 32 channels per chunk
+                    uint32_t v[32];
+                    tmem_ld32(t_row + chunk * 32, v);
+                    tmem_ld_wait();
+                    uint8_t *box_row = stg + (chunk >> 1) * (BM * 128) + row * 128;
+                    [[maybe_unused]] uint32_t q[8]; // e4m3: the chunk's 32 output bytes
 #pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    const int c16 = (chunk & 1) * 4 + j; // 16-byte column of the 128-byte row
-                    uint4 *cell = reinterpret_cast<uint4 *>(box_row + ((c16 ^ (row & 7)) << 4));
-                    const float4 b0 = *reinterpret_cast<const float4 *>(bias_s + wi.n_off + chunk * 32 + j * 8);
-                    const float4 b1 = *reinterpret_cast<const float4 *>(bias_s + wi.n_off + chunk * 32 + j * 8 + 4);
-                    float f[8];
-                    if constexpr (K::FP8) {
-                        const float4 d0 = *reinterpret_cast<const float4 *>(deq_s + wi.n_off + chunk * 32 + j * 8);
-                        const float4 d1 = *reinterpret_cast<const float4 *>(deq_s + wi.n_off + chunk * 32 + j * 8 + 4);
-                        const float d[8] = {d0.x, d0.y, d0.z, d0.w, d1.x, d1.y, d1.z, d1.w};
-                        const float b[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
+                    for (int j = 0; j < 4; ++j) {
+                        const int c16 = (chunk & 1) * 4 + j; // 16-byte column of the 128-byte row
+                        uint4 *cell = reinterpret_cast<uint4 *>(box_row + ((c16 ^ (row & 7)) << 4));
+                        const float4 b0 = *reinterpret_cast<const float4 *>(bias_s + wi.n_off + chunk * 32 + j * 8);
+                        const float4 b1 = *reinterpret_cast<const float4 *>(bias_s + wi.n_off + chunk * 32 + j * 8 + 4);
+                        float f[8];
+                        if constexpr (K::FP8) {
+                            const float4 d0 = *reinterpret_cast<const float4 *>(deq_s + wi.n_off + chunk * 32 + j * 8);
+                            const float4 d1 = *reinterpret_cast<const float4 *>(deq_s + wi.n_off + chunk * 32 + j * 8 + 4);
+                            const float d[8] = {d0.x, d0.y, d0.z, d0.w, d1.x, d1.y, d1.z, d1.w};
+                            const float b[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
 #pragma unroll
-                        for (int e = 0; e < 8; ++e) f[e] = fmaf(__uint_as_float(v[j * 8 + e]), d[e], b[e]);
-                    } else {
-                        f[0] = __uint_as_float(v[j * 8 + 0]) + b0.x; f[1] = __uint_as_float(v[j * 8 + 1]) + b0.y;
-                        f[2] = __uint_as_float(v[j * 8 + 2]) + b0.z; f[3] = __uint_as_float(v[j * 8 + 3]) + b0.w;
-                        f[4] = __uint_as_float(v[j * 8 + 4]) + b1.x; f[5] = __uint_as_float(v[j * 8 + 5]) + b1.y;
-                        f[6] = __uint_as_float(v[j * 8 + 6]) + b1.z; f[7] = __uint_as_float(v[j * 8 + 7]) + b1.w;
-                    }
-                    if (HAS_SKIP) {
-                        const uint4 sk = *cell;
-                        const uint32_t w[4] = {sk.x, sk.y, sk.z, sk.w};
+                            for (int e = 0; e < 8; ++e) f[e] = fmaf(__uint_as_float(v[j * 8 + e]), d[e], b[e]);
+                        } else {
+                            f[0] = __uint_as_float(v[j * 8 + 0]) + b0.x; f[1] = __uint_as_float(v[j * 8 + 1]) + b0.y;
+                            f[2] = __uint_as_float(v[j * 8 + 2]) + b0.z; f[3] = __uint_as_float(v[j * 8 + 3]) + b0.w;
+                            f[4] = __uint_as_float(v[j * 8 + 4]) + b1.x; f[5] = __uint_as_float(v[j * 8 + 5]) + b1.y;
+                            f[6] = __uint_as_float(v[j * 8 + 6]) + b1.z; f[7] = __uint_as_float(v[j * 8 + 7]) + b1.w;
+                        }
+                        if (HAS_SKIP) {
+                            const uint4 sk = *cell;
+                            const uint32_t w[4] = {sk.x, sk.y, sk.z, sk.w};
 #pragma unroll
-                        for (int e = 0; e < 4; ++e) {
-                            f[2 * e] += __uint_as_float(w[e] << 16);
-                            f[2 * e + 1] += __uint_as_float(w[e] & 0xFFFF0000u);
+                            for (int e = 0; e < 4; ++e) {
+                                f[2 * e] += __uint_as_float(w[e] << 16);
+                                f[2 * e + 1] += __uint_as_float(w[e] & 0xFFFF0000u);
+                            }
+                        }
+                        if constexpr (K::FP8) {
+#pragma unroll
+                            for (int e = 0; e < 8; ++e) f[e] = fmaxf(f[e], 0.f);
+                            if (qo.out_y) *cell = make_uint4(pack_bf16x2(f[0], f[1]), pack_bf16x2(f[2], f[3]), pack_bf16x2(f[4], f[5]),
+                                                             pack_bf16x2(f[6], f[7]));
+                            q[2 * j] = pack_e4m3x4(f[0] * inv_s, f[1] * inv_s, f[2] * inv_s, f[3] * inv_s);
+                            q[2 * j + 1] = pack_e4m3x4(f[4] * inv_s, f[5] * inv_s, f[6] * inv_s, f[7] * inv_s);
+                        } else {
+                            uint4 o;
+                            o.x = pack_bf16x2(fmaxf(f[0], 0.f), fmaxf(f[1], 0.f));
+                            o.y = pack_bf16x2(fmaxf(f[2], 0.f), fmaxf(f[3], 0.f));
+                            o.z = pack_bf16x2(fmaxf(f[4], 0.f), fmaxf(f[5], 0.f));
+                            o.w = pack_bf16x2(fmaxf(f[6], 0.f), fmaxf(f[7], 0.f));
+                            *cell = o;
                         }
                     }
                     if constexpr (K::FP8) {
-#pragma unroll
-                        for (int e = 0; e < 8; ++e) f[e] = fmaxf(f[e], 0.f);
-                        if (qo.out_y) *cell = make_uint4(pack_bf16x2(f[0], f[1]), pack_bf16x2(f[2], f[3]), pack_bf16x2(f[4], f[5]),
-                                                         pack_bf16x2(f[6], f[7]));
-                        q[2 * j] = pack_e4m3x4(f[0] * inv_s, f[1] * inv_s, f[2] * inv_s, f[3] * inv_s);
-                        q[2 * j + 1] = pack_e4m3x4(f[4] * inv_s, f[5] * inv_s, f[6] * inv_s, f[7] * inv_s);
-                    } else {
-                        uint4 o;
-                        o.x = pack_bf16x2(fmaxf(f[0], 0.f), fmaxf(f[1], 0.f));
-                        o.y = pack_bf16x2(fmaxf(f[2], 0.f), fmaxf(f[3], 0.f));
-                        o.z = pack_bf16x2(fmaxf(f[4], 0.f), fmaxf(f[5], 0.f));
-                        o.w = pack_bf16x2(fmaxf(f[6], 0.f), fmaxf(f[7], 0.f));
-                        *cell = o;
+                        if (qo.yq && q_row < qo.rows) {
+                            uint4 *dst = reinterpret_cast<uint4 *>(qo.yq + (size_t)q_row * C + wi.n_off + chunk * 32);
+                            dst[0] = make_uint4(q[0], q[1], q[2], q[3]);
+                            dst[1] = make_uint4(q[4], q[5], q[6], q[7]);
+                        }
                     }
                 }
-                if constexpr (K::FP8) {
-                    if (qo.yq && m0 + row < qo.rows) {
-                        uint4 *dst = reinterpret_cast<uint4 *>(qo.yq + (size_t)(m0 + row) * C + wi.n_off + chunk * 32);
-                        dst[0] = make_uint4(q[0], q[1], q[2], q[3]);
-                        dst[1] = make_uint4(q[4], q[5], q[6], q[7]);
-                    }
+                // accumulator buffer drained: hand it back to the MMA issuer
+                tc_fence_before();
+                __syncwarp();
+                if (lane == 0) {
+                    if constexpr (CG == 2) mbar_arrive_cluster(tempty0 + 8 * acc); else mbar_arrive(bar_tempty + 8 * acc);
                 }
+                if (++acc == 2) { acc = 0; acc_phase ^= 1; }
+                // staging tile -> global
+                fence_proxy_async();
+                asm volatile("bar.sync 1, 128;" ::: "memory");
+                if (threadIdx.x == 128) {
+                    bool store_y = true;
+                    if constexpr (K::FP8) store_y = qo.out_y != 0;
+                    if (store_y) {
+                        for (int g = 0; g < wi.n_w / 64; ++g) {
+                            if constexpr (PIX)
+                                tma_store_3d(&tm_y, staging + g * (BM * 128), wi.n_off + g * 64, tr.pix, tr.b0);
+                            else
+                                tma_store_2d(&tm_y, staging + g * (BM * 128), wi.n_off + g * 64, tr.m0);
+                        }
+                    }
+                    tma_store_commit();
+                    tma_store_wait_read();
+                    if (HAS_SKIP) mbar_arrive(bar_stfree);
+                }
+                asm volatile("bar.sync 1, 128;" ::: "memory");
             }
-            // accumulator buffer drained: hand it back to the MMA issuer
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) {
-                if constexpr (CG == 2) mbar_arrive_cluster(tempty0 + 8 * acc); else mbar_arrive(bar_tempty + 8 * acc);
-            }
-            if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-            // staging tile -> global
-            fence_proxy_async();
-            asm volatile("bar.sync 1, 128;" ::: "memory");
-            if (threadIdx.x == 128) {
-                bool store_y = true;
-                if constexpr (K::FP8) store_y = qo.out_y != 0;
-                if (store_y)
-                    for (int g = 0; g < wi.n_w / 64; ++g) tma_store_2d(&tm_y, staging + g * (BM * 128), wi.n_off + g * 64, m0);
-                tma_store_commit();
-                tma_store_wait_read();
-                if (HAS_SKIP) mbar_arrive(bar_stfree);
-            }
-            asm volatile("bar.sync 1, 128;" ::: "memory");
         }
         if (threadIdx.x == 128) tma_store_wait_all();
     }
@@ -690,14 +824,28 @@ inline bool encode_im2col(const Driver &d, CUtensorMap *m, const void *ptr, int 
                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-// d_count == nullptr: `n_tiles` cluster tiles planned here.  Otherwise the kernel plans from min(*d_count, count_cap)
-// boards on the device and every resident cluster is launched.
-template <int CG, int PAIRS, bool HAS_SKIP, bool DEV_COUNT, typename T = __nv_bfloat16>
+// NHWC activations [n,10,9,256] viewed as (channel, board pixel, board) for pixel tiles: box = one 128-byte row of
+// channels (64 bf16 / 128 e4m3) at one pixel of BM consecutive boards, 128-byte swizzle.  Boards past n read as zeros
+// and are not stored.
+inline bool encode_pixels(const Driver &d, CUtensorMap *m, const void *ptr, int n, bool e4m3 = false) {
+    const cuuint64_t esz = e4m3 ? 1 : 2;
+    const cuuint64_t dims[3] = {(cuuint64_t)C, (cuuint64_t)BOARD_HW, (cuuint64_t)n};
+    const cuuint64_t strides[2] = {(cuuint64_t)C * esz, (cuuint64_t)C * esz * BOARD_HW};
+    const cuuint32_t box[3] = {(cuuint32_t)(128 / esz), 1, BM};
+    const cuuint32_t es[3] = {1, 1, 1};
+    return d.tiled(m, e4m3 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void *>(ptr), dims, strides, box,
+                   es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+
+// d_count == nullptr: `n_units` scheduling units (conv_units) planned here.  Otherwise the kernel plans from
+// min(*d_count, count_cap) boards on the device and every resident cluster is launched.
+template <int CG, int PAIRS, bool HAS_SKIP, bool DEV_COUNT, typename T = __nv_bfloat16, bool PIX = false>
 inline cudaError_t launch_variant(const CUtensorMap &tx, const CUtensorMap &tw, const CUtensorMap &ts, const CUtensorMap &ty, const float *bias,
-                                  int n_tiles, int tail_split, int dbg, const int32_t *d_count, int count_cap, cudaStream_t stream,
+                                  int n_units, int tail_split, int dbg, const int32_t *d_count, int count_cap, cudaStream_t stream,
                                   const QOut<T> &qo = {}) {
     using K = Cfg<CG, T>;
-    auto kern = conv3x3_c256_kernel<CG, PAIRS, HAS_SKIP, DEV_COUNT, T>;
+    auto kern = conv3x3_c256_kernel<CG, PAIRS, HAS_SKIP, DEV_COUNT, T, PIX>;
     constexpr int CLUSTER = CG * PAIRS;
     // per device: resident clusters of this shape (GPC boundaries can strand SMs for CLUSTER > 2); function
     // attributes are per device too
@@ -734,7 +882,7 @@ inline cudaError_t launch_variant(const CUtensorMap &tx, const CUtensorMap &tw, 
         cfg.gridDim = dim3((unsigned)(max_clusters * CLUSTER));
         return cudaLaunchKernelEx(&cfg, kern, tx, tw, ts, ty, bias, 0, 0, 0, dbg, d_count, count_cap, tail_split, qo);
     }
-    const Plan pl = plan_items(n_tiles, max_clusters, tail_split != 0);
+    const Plan pl = plan_items(n_units, max_clusters, tail_split != 0);
     cfg.gridDim = dim3((unsigned)(pl.clusters * CLUSTER));
     return cudaLaunchKernelEx(&cfg, kern, tx, tw, ts, ty, bias, pl.n_items, pl.n_full, pl.split_log2, dbg, (const int32_t *)nullptr, 0, 0,
                               qo);

@@ -228,25 +228,27 @@ int ccz_replay_pack(const uint8_t *d_hist_boards /*[n,8,96]: history slots, most
  * in: y = relu(conv3x3_pad1(x, w) + bias [+ skip]) over n_boards boards of 10x9, 256 -> 256 channels.
  * d_x, d_skip, d_y: [n_boards,10,9,256] bf16 (NHWC = torch channels_last); d_w: [256][3][3][256] bf16
  * (out, kh, kw, in = a channels_last [256,256,3,3] weight); d_bias: fp32[256]; d_skip NULL = no skip
- * connection (conv1 of a block), d_skip may alias d_y but d_y must not alias d_x.  tcgen05 implicit GEMM
- * with TMA im2col loads.  variant 0 = the library default; otherwise bits 0-1 = CTA group (1: 128x256 tiles per
- * CTA, 2: CTA pairs on 256x256 tiles), bit 2 = no channel-sliced tail round, bits 5-6 = log2 of the CTA pairs
- * per cluster that share (multicast) one weight stage; bits 3-4 (skip every other weight / activation load:
- * WRONG results, energy-sensitivity measurements only) are rejected unless the library was built with
- * -DCCZ_CONV_EXPERIMENTS. */
+ * connection (conv1 of a block), d_skip may alias d_y but d_y must not alias d_x.  tcgen05 implicit GEMM.
+ * variant 0 = the library default = 128: pixel tiles (one board pixel x 256 boards per CTA pair, only the filter taps
+ * that fall on the board are multiplied).  Any other variant tiles consecutive NHWC pixels with TMA im2col loads (what
+ * variant 0 ran before pixel tiles; same results bit for bit): bits 0-1 = CTA group (1: 128x256 tiles per CTA, 2: CTA
+ * pairs on 256x256 tiles), bit 2 = no channel-sliced tail round, bits 5-6 = log2 of the CTA pairs per cluster that
+ * share (multicast) one weight stage; bits 3-4 (skip every other weight / activation load: WRONG results,
+ * energy-sensitivity measurements only) are rejected unless the library was built with -DCCZ_CONV_EXPERIMENTS. */
 int ccz_conv3x3_c256(const void *d_x, const void *d_w, const float *d_bias, const void *d_skip, void *d_y,
                      int n_boards, int variant, ccz_stream_t s);
 
 /* K9 over a board count that lives on the device: the buffers hold `capacity` boards (the tensor maps are encoded
  * for it) and the kernel convolves the first min(*d_n_boards, capacity) of them, planning its work items on the
  * device exactly as ccz_conv3x3_plan does for that count.  Every resident cluster is launched; clusters without an
- * item exit.  Output rows past the count (up to the end of the last tile) hold unspecified values.  Capture-safe: no
- * host synchronisation.  Each board's output is bit-identical to ccz_conv3x3_c256 over the same boards. */
+ * item exit.  Output rows past the count (up to the end of the last tile; with pixel tiles, every row of the boards up
+ * to the next multiple of 256) hold unspecified values.  Capture-safe: no host synchronisation.  Each board's output is bit-identical to ccz_conv3x3_c256 over the same boards. */
 int ccz_conv3x3_c256_count(const void *d_x, const void *d_w, const float *d_bias, const void *d_skip, void *d_y,
                            int capacity, const int32_t *d_n_boards, int variant, ccz_stream_t s);
 
-/* Host-only: the work plan ccz_conv3x3_c256 would launch for n_boards on a device with `resident_clusters`
- * co-resident clusters of the variant's shape (74 CTA pairs on a B200).  out[6] = {pixel rows per cluster tile,
+/* Host-only: the work plan ccz_conv3x3_c256 would launch for n_boards with tiles of consecutive pixels (variant 0 is read
+ * as 2, its CTA-pair shape) on a device with `resident_clusters` co-resident clusters of the variant's shape (74 CTA
+ * pairs on a B200).  out[6] = {pixel rows per cluster tile,
  * cluster tiles, work items, whole-tile items, log2 of the channel slices of the last partial round, clusters
  * launched}.  Work item i < out[3] is tile i over all 256 channels; item out[3] + j is channel slice
  * j % 2^out[4] (256 >> out[4] channels) of tile out[3] + (j >> out[4]); cluster c runs items c, c + out[5], ... */
@@ -298,10 +300,16 @@ int ccz_leaf_unique(const uint8_t *d_boards, int n, int32_t *d_rows, uint8_t *d_
  * graph follows a refreshed scale).  At least one output; neither output may alias d_xq, d_yq may not alias d_y or
  * d_skip; every pointer 16-byte aligned.  The buffers hold `capacity` boards; d_n_boards NULL = all of them, otherwise
  * the first min(*d_n_boards, capacity) as ccz_conv3x3_c256_count (each board's output is independent of its row, the
- * batch size and the work plan).  CTA pairs, channel-sliced tail round. */
+ * batch size and the work plan).  CTA pairs on tiles of consecutive pixels, channel-sliced tail round. */
 int ccz_conv3x3_c256_e4m3(const void *d_xq, const void *d_wq, const float *d_dequant, const float *d_bias, const void *d_skip,
                           void *d_y, void *d_yq, const float *d_inv_s_out, int capacity, const int32_t *d_n_boards,
                           ccz_stream_t s);
+
+/* ccz_conv3x3_c256_e4m3 with a tiling for A/B measurements: variant 0 = the default = 2 = tiles of consecutive pixels,
+ * 128 = pixel tiles as in ccz_conv3x3_c256 (same results bit for bit; slower in e4m3). */
+int ccz_conv3x3_c256_e4m3_variant(const void *d_xq, const void *d_wq, const float *d_dequant, const float *d_bias,
+                                  const void *d_skip, void *d_y, void *d_yq, const float *d_inv_s_out, int capacity,
+                                  const int32_t *d_n_boards, int variant, ccz_stream_t s);
 
 /* K10 with an e4m3 copy of its output: d_y as ccz_stem_lookup, d_yq e4m3 [n,10,9,256] = satfinite(d_y * *d_inv_s_out)
  * (the bf16 value, scaled in fp32).  d_n_boards NULL = all `capacity` boards, otherwise as ccz_stem_lookup_count. */
